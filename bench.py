@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: Apertis SSM+MoE block forward+backward tokens/s on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (ApertisLayer = pre-norm + SelectiveLinearAttention + residual,
 pre-norm + AdaptiveExpertSystem + residual; forward, synthetic loss of SURVEY.md 8(d), backward) over one
@@ -13,7 +13,17 @@ N > 1 (torchrun, one rank per GPU): experts sharded E/N per rank with NCCL all-t
 rank keeps its own batch (weak scaling), replicated-parameter gradients all-reduced as DDP would.
 
 --impl reference times the reference's algorithm on the host CPU: the oracle port (oracle/apertis_oracle.py,
-same ATen op sequence as core.py) with all host threads, on a bounded sample of the same workload.
+same ATen op sequence as core.py) with all host threads, on a bounded sample of the same workload, for --steps steps
+after --warmup warm-up steps.
+
+--dump-outputs DIR writes what the last timed step of the headline workload computed (rank 0) as DIR/<name>.npy in
+float32: the block output `out`, the aux losses `lb` and `rz`, `loss`, the input gradient `dx` and `grad.<parameter>`
+for every parameter.  A tensor of more than DUMP_SAMPLE elements is stored as the values at DUMP_SAMPLE sorted indices
+drawn with a fixed seed.  Weights, inputs, routing noise and dropout masks come from seeded generators: the same
+arguments give the same inputs in every run, so two builds can be compared output for output.  With N > 1 the
+gradients are rank 0's own, before the all-reduce of the replicated parameters (which the bench does into a separate
+buffer, not into .grad).  The outputs of the captured graph replayed last are kept alive for the dump, so later captures
+cannot reuse that memory: the work is the same, but the time of a dumping run is not strictly the time of a plain run.
 """
 import argparse
 import json
@@ -25,10 +35,12 @@ import tempfile
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the source tree may be read-only: nothing is cached next to it
 
 WORKLOADS = {
     # name: (Dm, H, I, E, K, seq)      shapes from SURVEY.md section 8 / BASELINE.md section 3
@@ -37,6 +49,30 @@ WORKLOADS = {
     "c4_7b": (1600, 25, 6400, 8, 2, 4096),
 }
 METRIC = "SSM+MoE block fwd+bwd tokens/sec"
+DUMP_SAMPLE = 1 << 20               # elements kept of one dumped tensor (4 MB in float32)
+DUMP_LIMIT = 64 << 20               # bytes of all dumped files together
+
+
+def dump_outputs(outputs, path):
+    """Writes {name: tensor} as path/<name>.npy (float32); larger tensors as a seeded sample of DUMP_SAMPLE elements."""
+    arrays, total = {}, 0
+    for name, t in outputs.items():
+        t = torch.as_tensor(t).detach()
+        flat = t.float().reshape(-1)
+        if flat.numel() > DUMP_SAMPLE:
+            g = torch.Generator().manual_seed(0)
+            idx = torch.randint(0, flat.numel(), (DUMP_SAMPLE,), generator=g).sort().values
+            flat = flat[idx.to(flat.device)]
+            a = flat.cpu().numpy()
+        else:
+            a = flat.cpu().numpy().reshape(tuple(t.shape))
+        arrays[name] = a
+        total += a.nbytes
+    if total > DUMP_LIMIT:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT}-byte limit")
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def peaks():
@@ -257,7 +293,13 @@ def main():
     ap.add_argument("--no-gpu-reference", action="store_true", help="skip timing the unmodified reference on the GPU")
     ap.add_argument("--graph", default="auto", choices=["auto", "on", "off"],
                     help="replay the step as a CUDA graph (auto: use it when capture and a replay check succeed)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last of them computed as DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs is not None:
+        ap.error("--dump-outputs writes what the B200 path computed; it does not apply to --impl reference")
     wl = WORKLOADS[args.workload]
     Dm, H, I, E, K, seq = wl
     rank = int(os.environ.get("RANK", "0"))
@@ -270,7 +312,7 @@ def main():
     if args.impl == "reference":
         if rank != 0:
             return
-        steps, warmup = max(1, min(args.steps, 5)), max(1, min(args.warmup, 2))
+        steps, warmup = args.steps, args.warmup
         v, ms, cores, sample, kind = cpu_reference_arm(args, wl, steps, warmup, args.cpu_sample_tokens)
         line = {"impl": "reference", "metric": METRIC, "value": v, "unit": "tokens/s", "n_gpus": args.gpus,
                 "steps": steps, "warmup": warmup, "ms_per_step": ms, "higher_is_better": True, "scaling": "weak",
@@ -300,7 +342,7 @@ def main():
 
     # headline: BASELINE.json configs[1] (the configuration the metric is quoted on) at every N, so the driver's
     # scaling series compares like with like
-    head = measure(args.workload, args.batch, ctx, clocks=True)
+    head = measure(args.workload, args.batch, ctx, clocks=True, dump_dir=args.dump_outputs)
     # configs[3] (7B-class, 8 experts top-2, experts sharded over the ranks) measured in the same run at every N
     extra = {}
     if not args.no_c4 and args.workload != "c4_7b":
@@ -391,9 +433,10 @@ def build_layer(name, ctx, dropout, ep=True):
     return layer.to(ctx["dev"]).train()
 
 
-def measure(name, B, ctx, clocks):
+def measure(name, B, ctx, clocks, dump_dir=None):
     """One workload on this rank's GPU: device-timed steps (CUDA graph replay when it captures), per-kernel times from an
-    eager pass, and the end-to-end loop with host inputs.  Times are the maximum over the ranks."""
+    eager pass, and the end-to-end loop with host inputs.  Times are the maximum over the ranks.  With `dump_dir`, what
+    the last timed step computed is written there (dump_outputs) before anything else runs."""
     import torch.distributed as dist
     from apertis_llm_b200 import _lib
     args, dev, world, rank = ctx["args"], ctx["dev"], ctx["world"], ctx["rank"]
@@ -406,8 +449,10 @@ def measure(name, B, ctx, clocks):
     dev_x = [h.to(dev, non_blocking=True).requires_grad_(True) for h in host_x]
     amp = args.dtype == "bf16"
     flat_grad = torch.zeros(sum(p.numel() for p in replicated), device=dev) if world > 1 else None
+    torch.manual_seed(4321 + rank)          # routing noise and dropout masks: the same draws in every run
 
-    def step(x):
+    def step(x, keep=None):
+        """keep: a dict that receives what the step hands its caller (detached: no autograd graph is held)."""
         for p in layer.parameters():
             p.grad = None
         x.grad = None
@@ -418,6 +463,9 @@ def measure(name, B, ctx, clocks):
         if world > 1:                                   # DDP-equivalent: one bucket of the replicated parameters' gradients
             torch._foreach_copy_(list(flat_grad.split([p.numel() for p in replicated])), [p.grad.reshape(-1) for p in replicated])
             dist.all_reduce(flat_grad)
+        if keep is not None:
+            keep.update(out=out.detach(), lb=lb.detach(), rz=rz.detach(), loss=loss.detach(), dx=x.grad)
+            keep.update({"grad." + n: p.grad for n, p in layer.named_parameters() if p.grad is not None})
         return loss
 
     def barrier():
@@ -446,10 +494,12 @@ def measure(name, B, ctx, clocks):
             graphs = []
             for i in range(nbuf):
                 g = torch.cuda.CUDAGraph()
+                # the graph replayed last keeps what its capture returned (a replay rewrites those tensors)
+                keep = {} if dump_dir is not None and i == (args.steps - 1) % nbuf else None
                 with torch.cuda.graph(g, pool=pool):
-                    gl = step(dev_x[i])
+                    gl = step(dev_x[i], keep)
                 pool = g.pool()
-                graphs.append((g, gl))
+                graphs.append((g, gl, keep))
             barrier()
             eager = float(step(dev_x[0]).detach())
             graphs[0][0].replay()
@@ -463,11 +513,11 @@ def measure(name, B, ctx, clocks):
                 raise
             barrier()
 
-    def run_step(i):
+    def run_step(i, keep=None):
         if graphs is not None:
             graphs[i % nbuf][0].replay()
             return graphs[i % nbuf][1]
-        return step(dev_x[i % nbuf])
+        return step(dev_x[i % nbuf], keep)
 
     # ---- timed region: device-resident inputs, CUDA events
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -484,15 +534,18 @@ def measure(name, B, ctx, clocks):
         if graphs is None:
             launches0 = _lib.launch_count
             _lib.start_timing(TIMED)
+        last = {} if dump_dir is not None else None
         e0.record()
         for i in range(args.steps):
-            run_step(i)
+            run_step(i, last if i == args.steps - 1 else None)
         e1.record()
         barrier()
         if graphs is None:
             per_kernel = _lib.stop_timing()
             launches = _lib.launch_count - launches0
     ms = e0.elapsed_time(e1) / args.steps
+    if dump_dir is not None and rank == 0:
+        dump_outputs(graphs[(args.steps - 1) % nbuf][2] if graphs is not None else last, dump_dir)
     clk_summary = clk.summary()
     if graphs is not None:
         # per-kernel CUDA events cannot be read inside a replayed graph: the same steps once more, eagerly, for the

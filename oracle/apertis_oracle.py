@@ -251,7 +251,7 @@ def moe_forward(p: Params, x: Tensor, *, E: int, K: int, eps: float = 1e-12,
     cap = moe_capacity(S, E, cap_factor, training, use_capacity)            # :508-511
     if training and rz_coef > 0:                                            # :524-526
         rz = rz_coef * torch.mean(torch.logsumexp(logits, dim=-1) ** 2)
-    kept, counts, groups = moe_plan(idx.numpy(), w.detach().numpy(), E, cap, active,
+    kept, counts, groups = moe_plan(idx.cpu().numpy(), w.detach().cpu().numpy(), E, cap, active,
                                     limit=(use_capacity and training))
     out = torch.zeros_like(x2)                                              # :531
     fn = _act(act)
@@ -260,7 +260,7 @@ def moe_forward(p: Params, x: Tensor, *, E: int, K: int, eps: float = 1e-12,
             take = groups.get((k, e))
             if take is None:
                 continue
-            rows = torch.from_numpy(take)
+            rows = torch.from_numpy(take).to(x2.device)
             xe = x2[rows]                                                   # :593
             h = F.layer_norm(xe, (Dm,), p[f"experts.{e}.0.weight"], p[f"experts.{e}.0.bias"], eps)
             h = fn(F.linear(h, p[f"experts.{e}.1.weight"], p[f"experts.{e}.1.bias"]))

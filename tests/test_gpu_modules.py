@@ -317,35 +317,26 @@ def test_cuda_graph_replay_matches_eager(Dm):
             assert rel_err(v, eager_g[k]) < 1e-2, k
 
 
+# the unmodified reference's own bf16-autocast deviation at C4 dims on a B200 reached 4.7 % on the router-path gradients
+# (DESIGN.md section 2); no bf16 bound below may be wider than twice that
+REFERENCE_BF16_FLOOR_MAX = 0.047
+
+
 def reference_bf16_floor(spec, sd, x, noise, want):
-    """The error the UNMODIFIED reference layer (baseline/_ref) makes on this GPU under bf16 autocast, on the same weights,
-    inputs and routing noise, against the fp32 gradients `want` (metric: tests.util.rel_err per tensor).  It is the noise
-    floor of a bf16 run of this shape: near-tied tokens re-route, sums over tokens cancel.  {} when the reference is absent."""
-    from baseline import ref_loader
-    if not ref_loader.available():
-        return {}
-    core = ref_loader.load_core()
-    cfg = core.ApertisConfig(hidden_size=spec["Dm"], num_attention_heads=spec["H"], intermediate_size=spec["I"],
-                             num_hidden_layers=1, attention_type="selective_ssm", use_expert_system=True,
-                             num_experts=spec["E"], experts_per_token=spec["K"], vocab_size=64, hidden_dropout_prob=0.0,
-                             attention_probs_dropout_prob=0.0, hidden_act=spec.get("act", "gelu"))
-    ref = core.ApertisLayer(cfg)
-    missing, unexpected = ref.load_state_dict(sd, strict=False)
-    assert not unexpected, unexpected
-    ref = ref.to(dev()).train()
-    nz = noise.to(dev())
-    orig = torch.randn_like
-    torch.randn_like = lambda t, *a, **k: nz.to(t.dtype) if tuple(t.shape) == tuple(nz.shape) else orig(t, *a, **k)
-    try:
-        xr = x.to(dev()).requires_grad_(True)
-        with torch.autocast("cuda", dtype=torch.bfloat16):
-            out, _, _, lb, rz = ref(xr)
-        O.block_loss(out.float(), lb.float(), rz.float()).backward()
-    finally:
-        torch.randn_like = orig
+    """The error a bf16-autocast run of the reference's algorithm makes on this GPU, on the same weights, inputs and routing
+    noise, against the fp32 gradients `want` (metric: tests.util.rel_err per tensor): the noise floor of a bf16 run of this
+    shape, where near-tied tokens re-route and sums over tokens cancel.  The layer run is the oracle (the reference layer's
+    op sequence, pinned to the reference in fp32 by tests/test_oracle_golden.py).  Its bf16 deviation is not the
+    reference's: at C4 dims it runs up to 10 % on the router-path gradients where the reference's stayed within 4.7 %, so
+    the caller caps it at REFERENCE_BF16_FLOOR_MAX."""
+    sdg = {k: v.to(dev()).requires_grad_(True) for k, v in sd.items()}
+    with torch.autocast("cuda", dtype=torch.bfloat16):
+        out, lb, rz = O.block_forward(sdg, x.to(dev()), num_heads=spec["H"], E=spec["E"], K=spec["K"], training=True,
+                                      noise=noise.to(dev()), act=spec.get("act", "gelu"))
+    O.block_loss(out.float(), lb.float(), rz.float()).backward()
     torch.cuda.synchronize()
-    floor = {k: rel_err(p.grad, want[k]) for k, p in ref.named_parameters() if p.grad is not None and k in want}
-    del ref
+    floor = {k: rel_err(p.grad, want[k]) for k, p in sdg.items() if p.grad is not None and k in want}
+    del sdg, out
     torch.cuda.empty_cache()
     return floor
 
@@ -412,12 +403,13 @@ def test_block_baseline_configs_vs_oracle(name, Dm, H, I, B, L, autocast):
         dg, dr = xg.grad.reshape(S, Dm).cpu().double(), xr.grad.reshape(S, Dm).double()
         assert float((dg - dr).norm() / dr.norm()) < 2e-2, "dx"
     # bf16: parameter gradients are sums over all tokens in which re-routed tokens and cancellation show; the bound is 5e-2
-    # or twice what the unmodified reference's own bf16-autocast run on this GPU deviates from the same fp32 gradients
+    # or twice what a bf16-autocast run of the reference's algorithm on this GPU deviates from the same fp32 gradients,
+    # that deviation capped at the largest one recorded for the unmodified reference
     floor = reference_bf16_floor(spec, sd, x, noise, {k: v.grad for k, v in sdr.items()}) if autocast else {}
     bad = []
     for k, gr in named_grads(layer).items():
         e = rel_err(gr, sdr[k].grad)
-        bound = tol if not autocast else max(5e-2, 2.0 * floor.get(k, 0.0))
+        bound = tol if not autocast else max(5e-2, 2.0 * min(floor.get(k, 0.0), REFERENCE_BF16_FLOOR_MAX))
         if not e < bound:
             bad.append((k, round(e, 4), floor.get(k)))
     assert not bad, "(tensor, error, reference bf16 floor): " + "; ".join(map(str, bad))

@@ -1,25 +1,22 @@
-"""patch_apertis_model against the UNMODIFIED reference model (build container only: /root/reference is absent on the
-GPU box, where this file skips).  CPU-only: checks the module swap, parameter adoption and state_dict compatibility;
-the numerical parity of the swapped modules is what tests/test_gpu_modules.py covers through the golden vectors."""
-import os
-import sys
-
+"""patch_apertis_model against the UNMODIFIED reference model (baseline/_ref, installed by __graft_entry__.build() where a
+reference checkout is at hand; the file skips without it).  CPU-only: checks the module swap, parameter adoption and
+state_dict compatibility; the numerical parity of the swapped modules is what tests/test_gpu_modules.py covers through
+the golden vectors."""
 import pytest
 import torch
 
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "src", "model")), reason="reference checkout not present")
+from baseline import ref_loader
+
+pytestmark = pytest.mark.skipif(not ref_loader.available(), reason="baseline/_ref (the installed reference) is absent")
 
 
 def _ref_model():
-    if REF not in sys.path:
-        sys.path.insert(0, REF)
-    from src.model.core import ApertisConfig, ApertisForCausalLM
-    cfg = ApertisConfig(hidden_size=64, num_attention_heads=4, intermediate_size=128, num_hidden_layers=2,
-                        attention_type="selective_ssm", use_expert_system=True, num_experts=4, experts_per_token=2,
-                        vocab_size=97, hidden_dropout_prob=0.0, attention_probs_dropout_prob=0.0)
+    core = ref_loader.load_core()
+    cfg = core.ApertisConfig(hidden_size=64, num_attention_heads=4, intermediate_size=128, num_hidden_layers=2,
+                             attention_type="selective_ssm", use_expert_system=True, num_experts=4, experts_per_token=2,
+                             vocab_size=97, hidden_dropout_prob=0.0, attention_probs_dropout_prob=0.0)
     torch.manual_seed(0)
-    return ApertisForCausalLM(cfg)
+    return core.ApertisForCausalLM(cfg)
 
 
 def test_patch_swaps_modules_and_keeps_state_dict():
