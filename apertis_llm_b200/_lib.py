@@ -165,7 +165,7 @@ KERNELS_PER_CALL = {
     "ab_selective_scan_fwd": 1, "ab_selective_scan_bwd": 2,          # single pass; two pass adds 2
     "ab_ssm_scan_fwd": 1, "ab_ssm_scan_bwd": 2, "ab_dense_gemm_nt": 1, "ab_dense_gemm_nn": 1, "ab_dense_gemm_tn": 2,
     "ab_dt_compose_fwd": 1, "ab_dt_compose_bwd": 2,
-    "ab_moe_router_fwd": 2, "ab_moe_topk_from_logits": 1, "ab_moe_plan": 2, "ab_moe_permute_ln": 1, "ab_moe_unpermute": 1,
+    "ab_moe_router_fwd": 2, "ab_moe_topk_from_logits": 1, "ab_moe_plan": 7, "ab_moe_permute_ln": 1, "ab_moe_unpermute": 1,
     "ab_moe_unpermute_bwd": 1, "ab_moe_permute_ln_bwd": 2, "ab_moe_segment_colsum": 2, "ab_moe_router_bwd": 3,
     "ab_layernorm_fwd": 1, "ab_layernorm_bwd": 3,
     "ab_grouped_gemm_nt": 1, "ab_grouped_gemm_nn": 1, "ab_grouped_gemm_tn": 1, "ab_cast_f32_to_bf16": 1,

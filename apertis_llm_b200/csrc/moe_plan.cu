@@ -46,73 +46,59 @@ __device__ __forceinline__ void st4(T* p, float a, float b, float c, float d) {
     }
 }
 
-constexpr int PLAN_THREADS = 1024;
+// Capacity plan over the whole GPU, in four steps that each read idx / w once (launch order = dependency order):
+//   (1) plan_hist_kernel, pass 3..0: per (expert, slot) 256-bin histograms of one byte of the weight bits of the candidates
+//       that still match the threshold prefix found so far.  The last CTA to finish (atomic ticket) turns the global
+//       histograms into the next byte of the threshold; after pass 3 it also fixes each slot's mode and base from the
+//       candidate counts: slot k is filled before slot k+1 with the remaining capacity.
+//   (2) plan_chunk_count_kernel: per chunk of PLAN_CHUNK tokens and (expert, slot), the candidates above the threshold
+//       ("gt") and equal to it ("eq").
+//   (3) plan_pos_kernel: a kept (token, slot) sits at base + gt before it + min(eq before it, eq taken): ties at the
+//       threshold are taken in token order.  Each CTA adds the counts of the chunks before its own.  Same result as one CTA walking the tokens of each expert in order.
+constexpr int PLAN_THREADS = 256;
+constexpr int PLAN_CHUNK = PLAN_THREADS;     // tokens per CTA of steps (2) and (3): one per thread
+constexpr int HIST_TOKENS = PLAN_THREADS;    // tokens per CTA of step (1): one per thread, loads all in flight at once
 
-// exclusive prefix of a small per-thread count over the CTA (thread order) + CTA total; two __syncthreads
-__device__ __forceinline__ int block_excl_scan(int cnt, int* warp_tot /*[32]*/, int& total) {
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    int inc = cnt;
+// per (expert, slot) state written by the last CTA of each histogram pass
+struct PlanSel {
+    uint32_t prefix;   // threshold bits found so far (then the threshold itself)
+    int need;          // elements equal to the threshold that are still to be taken
+    int mode;          // 0 none, 1 all, 2 select the `need` largest
+    int base;          // kept rows of the expert in earlier slots
+};
+
+// From a 256-bin histogram, by one warp: the bin holding the `need`-th largest element counted from the top, and how many
+// are still needed inside it.  Lane l owns bins [8l, 8l+8); suffix sums over the lanes by shuffles.
+__device__ __forceinline__ void warp_select_bin(const int* hist, int lane, int& need, int& sel_bin) {
+    int h[8], mine = 0;
+#pragma unroll
+    for (int i = 0; i < 8; ++i) { h[i] = hist[lane * 8 + i]; mine += h[i]; }
+    int incl = mine;
 #pragma unroll
     for (int o = 1; o < 32; o <<= 1) {
-        const int v = __shfl_up_sync(0xffffffffu, inc, o);
-        if (lane >= o) inc += v;
+        const int v = __shfl_down_sync(0xffffffffu, incl, o);
+        if (lane + o < 32) incl += v;
     }
-    if (lane == 31) warp_tot[warp] = inc;
-    __syncthreads();
-    int before = 0, tot = 0;
-    const int nw = blockDim.x >> 5;
-    for (int i = 0; i < nw; ++i) {
-        const int c = warp_tot[i];
-        if (i < warp) before += c;
-        tot += c;
-    }
-    __syncthreads();
-    total = tot;
-    return before + inc - cnt;
-}
-
-// One CTA per expert.  row_local[s,k] = position of the kept (token, slot) inside the expert's segment, -1 if dropped.
-// Per slot: (A) the expert's candidates are compacted in token order into a shared-memory list (token id, weight bits)
-// while the top-byte histogram is built; (B) on overflow of the capacity the rem-th largest weight is radix-selected on
-// the list; (C) positions are assigned in list (= token) order.  If the candidates do not fit the list the slot falls
-// back to the same algorithm over global memory.
-constexpr int TPT = 8;   // consecutive tokens per thread per compaction sweep
-
-// From a 256-bin histogram: the bin holding the `need`-th largest element counted from the top, and how many are still needed
-// inside it.  Warp 0: lane l owns bins [8l, 8l+8); suffix sums over the lanes by shuffles instead of a 256-step serial scan.
-__device__ __forceinline__ void radix_select_bin(int* hist, int& need, int& sel_bin, int* s_sel_bin, int* s_need) {
-    if (threadIdx.x < 32) {
-        const int lane = threadIdx.x;
-        int h[8], mine = 0;
-#pragma unroll
-        for (int i = 0; i < 8; ++i) { h[i] = hist[lane * 8 + i]; mine += h[i]; }
-        // elements in the bins of higher lanes: inclusive suffix scan by shuffles, minus the lane's own count
-        int incl = mine;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const int v = __shfl_down_sync(0xffffffffu, incl, o);
-            if (lane + o < 32) incl += v;
+    const int above = incl - mine;
+    const int nd0 = need;
+    const bool here = above < nd0 && above + mine >= nd0;       // the wanted element lies in this lane's bins
+    const unsigned who = __ballot_sync(0xffffffffu, here);
+    int bin = 0, nd = 0;
+    if (who == 0u) {                                            // fewer than `need` elements in total: lowest bin
+        nd = __shfl_sync(0xffffffffu, nd0 - (above + mine) + h[0], 0);
+        bin = 0;
+    } else {
+        const int src = __ffs(who) - 1;
+        int b = 7, n2 = nd0 - above;
+        for (; b > 0; --b) {
+            if (h[b] >= n2) break;
+            n2 -= h[b];
         }
-        const int above = incl - mine;
-        const int nd0 = need;
-        const bool here = above < nd0 && above + mine >= nd0;       // the wanted element lies in this lane's bins
-        const unsigned who = __ballot_sync(0xffffffffu, here);
-        if (who == 0u) {                                            // fewer than `need` elements in total: lowest bin
-            if (lane == 0) { *s_sel_bin = 0; *s_need = nd0 - (above + mine) + h[0]; }
-        } else if (lane == __ffs(who) - 1) {
-            int nd = nd0 - above, bin = 7;
-            for (; bin > 0; --bin) {
-                if (h[bin] >= nd) break;
-                nd -= h[bin];
-            }
-            *s_sel_bin = lane * 8 + bin;
-            *s_need = nd;
-        }
+        bin = __shfl_sync(0xffffffffu, lane * 8 + b, src);
+        nd = __shfl_sync(0xffffffffu, n2, src);
     }
-    __syncthreads();
-    sel_bin = *s_sel_bin;
-    need = *s_need;
-    __syncthreads();
+    sel_bin = bin;
+    need = nd;
 }
 
 // histogram increment with one shared-memory atomic per distinct bin per warp: gate weights share their top bytes, so
@@ -125,129 +111,175 @@ __device__ __forceinline__ void hist_add_warp(int* hist, bool valid, int bin) {
     }
 }
 
-__global__ void __launch_bounds__(PLAN_THREADS) plan_count_kernel(const int32_t* __restrict__ idx, const float* __restrict__ w,
-                                                                  const int32_t* __restrict__ active, int cap,
-                                                                  int32_t* __restrict__ counts, int32_t* __restrict__ row_local,
-                                                                  int S, int K, int list_cap) {
-    extern __shared__ uint2 s_list[];          // [list_cap] (token, weight bits) of the current slot's candidates
-    __shared__ int hist[256];
-    __shared__ int warp_tot[32];
-    __shared__ int s_sel_bin, s_need;
-    const int e = blockIdx.x;
-    const int tid = threadIdx.x;
-    const bool is_active = active == nullptr || active[e] != 0;
-    int kept_total = 0;
-    for (int k = 0; k < K; ++k) {
-        // ---- (A) compaction in token order (histograms are only built when the capacity overflows, in (B))
-        int n_cand = 0;
-        const int span = blockDim.x * TPT;
-        for (int s0 = 0; s0 < S; s0 += span) {
-            const int sb = s0 + tid * TPT;
-            uint32_t wb[TPT];
-            bool c[TPT];
-            int mine = 0;
-#pragma unroll
-            for (int t = 0; t < TPT; ++t) {
-                const int s = sb + t;
-                c[t] = s < S && idx[(size_t)s * K + k] == e;
-                wb[t] = c[t] ? __float_as_uint(w[(size_t)s * K + k]) : 0u;
-                mine += c[t];
+// true in exactly one CTA of the grid, the last to get here, after all others' global writes are visible
+__device__ __forceinline__ bool last_cta(int* ticket) {
+    __shared__ bool s_last;
+    __threadfence();
+    __syncthreads();
+    if (threadIdx.x == 0) s_last = atomicAdd(ticket, 1) == (int)(gridDim.x * gridDim.y) - 1;
+    __syncthreads();
+    if (s_last) __threadfence();
+    return s_last;
+}
+
+// grid (ceil(S / HIST_TOKENS), K): slot k = blockIdx.y.  hist: [E*K][256] of this pass, zeroed by the caller.
+__global__ void __launch_bounds__(PLAN_THREADS) plan_hist_kernel(const int32_t* __restrict__ idx, const float* __restrict__ w,
+                                                                 const int32_t* __restrict__ active, int cap, int pass,
+                                                                 int* __restrict__ ghist, PlanSel* __restrict__ sel,
+                                                                 int* __restrict__ any_select, int* __restrict__ ticket,
+                                                                 int32_t* __restrict__ counts, int S, int K, int E) {
+    __shared__ int hist[32 * 256];
+    if (pass < 3 && *any_select == 0) return;                  // uniform over the grid: no slot overflows its capacity
+    const int k = blockIdx.y, tid = threadIdx.x;
+    for (int i = tid; i < E * 256; i += blockDim.x) hist[i] = 0;
+    __syncthreads();
+    const int shift = 8 * pass;
+    const uint32_t mask = pass == 3 ? 0u : 0xffffffffu << (shift + 8);
+    const int s_end = min(S, (int)(blockIdx.x + 1) * HIST_TOKENS);
+    for (int s0 = blockIdx.x * HIST_TOKENS; s0 < s_end; s0 += blockDim.x) {
+        const int s = s0 + tid;
+        bool c = s < s_end;
+        int e = 0;
+        uint32_t b = 0u;
+        if (c) {
+            e = idx[(size_t)s * K + k];
+            b = __float_as_uint(w[(size_t)s * K + k]);
+            if (pass < 3) {
+                const PlanSel st = sel[e * K + k];
+                c = st.mode == 2 && (b & mask) == st.prefix;
             }
-            int tot;
-            int pos = n_cand + block_excl_scan(mine, warp_tot, tot);
-#pragma unroll
-            for (int t = 0; t < TPT; ++t) {
-                if (c[t]) {
-                    if (pos < list_cap) s_list[pos] = make_uint2((uint32_t)(sb + t), wb[t]);
-                    ++pos;
-                }
-            }
-            n_cand += tot;
         }
-        __syncthreads();
-        const bool in_smem = n_cand <= list_cap;
-        const int rem = cap - kept_total;
-        int mode = 0;                       // 0 none, 1 all, 2 select the `rem` largest
-        if (is_active && n_cand > 0 && rem > 0) mode = n_cand <= rem ? 1 : 2;
-        uint32_t tau = 0;
-        int n_eq_take = 0;
-        if (mode == 2) {
-            // ---- (B) radix select of the rem-th largest weight (positive floats order like their bit patterns)
-            uint32_t prefix = 0, mask = 0;
-            int need = rem, bin;
-            for (int pass = 3; pass >= 0; --pass) {
-                for (int i = tid; i < 256; i += blockDim.x) hist[i] = 0;
-                __syncthreads();
-                if (in_smem) {
-                    for (int i0 = 0; i0 < n_cand; i0 += blockDim.x) {
-                        const int i = i0 + tid;
-                        const uint32_t b = i < n_cand ? s_list[i].y : 0u;
-                        hist_add_warp(hist, i < n_cand && (b & mask) == prefix, (int)((b >> (8 * pass)) & 0xff));
-                    }
-                } else {
-                    for (int s0 = 0; s0 < S; s0 += blockDim.x) {
-                        const int s = s0 + tid;
-                        const bool c = s < S && idx[(size_t)s * K + k] == e;
-                        const uint32_t b = c ? __float_as_uint(w[(size_t)s * K + k]) : 0u;
-                        hist_add_warp(hist, c && (b & mask) == prefix, (int)((b >> (8 * pass)) & 0xff));
-                    }
-                }
-                __syncthreads();
-                radix_select_bin(hist, need, bin, &s_sel_bin, &s_need);
-                prefix |= (uint32_t)bin << (8 * pass);
-                mask |= 0xffu << (8 * pass);
-            }
-            tau = prefix;
-            n_eq_take = need;
-        }
-        // ---- (C) positions in token order
-        int run_eq = 0, run_kept = 0;
-        const int n_items = in_smem ? n_cand : S;
-        for (int s0 = 0; s0 < n_items; s0 += span) {
-            const int ib = s0 + tid * TPT;
-            bool c[TPT], gt[TPT], eq[TPT];
-            int tokv[TPT];
-            int n_eq = 0;
-#pragma unroll
-            for (int t = 0; t < TPT; ++t) {
-                const int i = ib + t;
-                uint32_t b = 0u;
-                if (in_smem) {
-                    c[t] = i < n_cand;
-                    if (c[t]) { const uint2 it = s_list[i]; tokv[t] = (int)it.x; b = it.y; } else tokv[t] = 0;
-                } else {
-                    c[t] = i < S && idx[(size_t)i * K + k] == e;
-                    tokv[t] = i;
-                    if (c[t]) b = __float_as_uint(w[(size_t)i * K + k]);
-                }
-                gt[t] = c[t] && (mode == 1 || (mode == 2 && b > tau));
-                eq[t] = c[t] && mode == 2 && b == tau;
-                n_eq += eq[t];
-            }
-            int tot_eq = 0, tot_kept = 0;
-            int eq_rank = run_eq;
-            if (mode == 2) eq_rank += block_excl_scan(n_eq, warp_tot, tot_eq);
-            bool kept[TPT];
-            int n_kept = 0;
-#pragma unroll
-            for (int t = 0; t < TPT; ++t) {
-                kept[t] = gt[t] || (eq[t] && eq_rank < n_eq_take);
-                eq_rank += eq[t];
-                n_kept += kept[t];
-            }
-            int pos = kept_total + run_kept + block_excl_scan(n_kept, warp_tot, tot_kept);
-#pragma unroll
-            for (int t = 0; t < TPT; ++t) {
-                if (c[t]) row_local[(size_t)tokv[t] * K + k] = kept[t] ? pos : -1;
-                pos += kept[t];
-            }
-            run_eq += tot_eq;
-            run_kept += tot_kept;
-        }
-        kept_total += run_kept;
-        __syncthreads();
+        hist_add_warp(hist, c, e * 256 + (int)((b >> shift) & 0xffu));
     }
-    if (tid == 0) counts[e] = kept_total;
+    __syncthreads();
+    int* gh = ghist + (size_t)k * 256;                         // [E][K][256]: expert e, slot k at (e*K + k)*256
+    for (int i = tid; i < E * 256; i += blockDim.x) {
+        const int h = hist[i];
+        if (h) atomicAdd(&gh[(size_t)(i >> 8) * K * 256 + (i & 255)], h);
+    }
+    if (!last_cta(ticket)) return;
+    // ---- last CTA: one warp per expert
+    const int lane = tid & 31, warp = tid >> 5;
+    int any = 0;
+    for (int e = warp; e < E; e += blockDim.x >> 5) {
+        int kept = 0;
+        for (int kk = 0; kk < K; ++kk) {
+            const int* hk = ghist + ((size_t)e * K + kk) * 256;
+            PlanSel st;
+            if (pass == 3) {
+                int n = 0;
+                for (int i = lane; i < 256; i += 32) n += hk[i];
+                n = __reduce_add_sync(0xffffffffu, n);
+                const bool is_active = active == nullptr || active[e] != 0;
+                const int rem = cap - kept;
+                st.mode = 0;
+                if (is_active && n > 0 && rem > 0) st.mode = n <= rem ? 1 : 2;
+                st.base = kept;
+                st.need = rem;
+                st.prefix = 0u;
+                kept += st.mode == 1 ? n : (st.mode == 2 ? rem : 0);
+            } else {
+                st = sel[e * K + kk];
+            }
+            if (st.mode == 2) {
+                int bin;
+                warp_select_bin(hk, lane, st.need, bin);
+                st.prefix |= (uint32_t)bin << shift;
+                any = 1;
+            }
+            if (lane == 0) sel[e * K + kk] = st;
+        }
+        if (pass == 3 && lane == 0) counts[e] = kept;
+    }
+    if (pass == 3) {
+        __shared__ int s_any;
+        if (tid == 0) s_any = 0;
+        __syncthreads();
+        if (any && lane == 0) s_any = 1;
+        __syncthreads();
+        if (tid == 0) *any_select = s_any;
+    }
+}
+
+// the class of a candidate under its slot's threshold: 0 above it (or mode 1), 1 equal (mode 2), -1 not kept
+__device__ __forceinline__ int plan_class(const PlanSel& st, uint32_t b) {
+    if (st.mode == 1) return 0;
+    if (st.mode == 2) return b > st.prefix ? 0 : (b == st.prefix ? 1 : -1);
+    return -1;
+}
+
+// grid (ceil(S / PLAN_CHUNK), K).  cc: [chunks][K][E][2] candidates above / equal to the threshold per chunk
+__global__ void __launch_bounds__(PLAN_THREADS) plan_chunk_count_kernel(const int32_t* __restrict__ idx, const float* __restrict__ w,
+                                                                        const PlanSel* __restrict__ sel, int* __restrict__ cc,
+                                                                        int S, int K, int E) {
+    __shared__ int cnt[64];
+    const int k = blockIdx.y, tid = threadIdx.x;
+    if (tid < 2 * E) cnt[tid] = 0;
+    __syncthreads();
+    const int s = blockIdx.x * PLAN_CHUNK + tid;
+    int cls = -1, e = 0;
+    if (s < S) {
+        e = idx[(size_t)s * K + k];
+        cls = plan_class(sel[e * K + k], __float_as_uint(w[(size_t)s * K + k]));
+    }
+    hist_add_warp(cnt, cls >= 0, e * 2 + (cls > 0 ? 1 : 0));
+    __syncthreads();
+    if (tid < 2 * E) cc[((size_t)blockIdx.x * K + k) * 2 * E + tid] = cnt[tid];
+}
+
+// grid (ceil(S / PLAN_CHUNK), K): row_local[s,k] = position of the kept (token, slot) inside the expert's segment, -1 if dropped
+__global__ void __launch_bounds__(PLAN_THREADS) plan_pos_kernel(const int32_t* __restrict__ idx, const float* __restrict__ w,
+                                                                const PlanSel* __restrict__ sel, const int* __restrict__ cc,
+                                                                int32_t* __restrict__ row_local, int S, int K, int E) {
+    __shared__ int wcnt[PLAN_THREADS / 32][64];                // per warp: [e][gt, eq], then their exclusive prefix over warps
+    __shared__ int sbase[PLAN_THREADS];
+    const int k = blockIdx.y, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    // counts of the earlier chunks: column (e, gt|eq) = tid % 2E, chunk groups interleaved over the rest of the threads
+    {
+        const int ncol = 2 * E, ng = PLAN_THREADS / ncol, col = tid % ncol, grp = tid / ncol;
+        int sum = 0;
+        if (grp < ng)
+            for (int c = grp; c < (int)blockIdx.x; c += ng) sum += cc[((size_t)c * K + k) * ncol + col];
+        sbase[tid] = sum;
+    }
+    const int s = blockIdx.x * PLAN_CHUNK + tid;
+    int cls = -1, e = 0;
+    PlanSel st{0u, 0, 0, 0};
+    if (s < S) {
+        e = idx[(size_t)s * K + k];
+        st = sel[e * K + k];
+        cls = plan_class(st, __float_as_uint(w[(size_t)s * K + k]));
+    }
+    const unsigned valid = __ballot_sync(0xffffffffu, s < S);
+    const unsigned same = __match_any_sync(0xffffffffu, s < S ? e : -1) & valid;
+    const unsigned gtm = __ballot_sync(0xffffffffu, cls == 0), eqm = __ballot_sync(0xffffffffu, cls == 1);
+    const unsigned lt = (1u << lane) - 1u;
+    for (int i = tid; i < (PLAN_THREADS / 32) * 64; i += blockDim.x) (&wcnt[0][0])[i] = 0;
+    __syncthreads();
+    if (s < S && (__ffs(same) - 1) == lane) {
+        wcnt[warp][2 * e] = __popc(same & gtm);
+        wcnt[warp][2 * e + 1] = __popc(same & eqm);
+    }
+    __syncthreads();
+    if (tid < 2 * E) {
+        int run = 0;
+        for (int g = 0; g < PLAN_THREADS / (2 * E); ++g) run += sbase[g * 2 * E + tid];
+        for (int wv = 0; wv < PLAN_THREADS / 32; ++wv) {
+            const int v = wcnt[wv][tid];
+            wcnt[wv][tid] = run;
+            run += v;
+        }
+    }
+    __syncthreads();
+    if (s < S) {
+        int r = -1;
+        if (cls >= 0) {
+            const int gt_before = wcnt[warp][2 * e] + __popc(same & gtm & lt);
+            const int eq_before = wcnt[warp][2 * e + 1] + __popc(same & eqm & lt);
+            if (cls == 0 || eq_before < st.need) r = st.base + gt_before + min(eq_before, st.need);
+        }
+        row_local[(size_t)s * K + k] = r;
+    }
 }
 
 __global__ void plan_finalize_kernel(const int32_t* __restrict__ idx, const int32_t* __restrict__ counts,
@@ -748,10 +780,23 @@ extern "C" int64_t ab_moe_max_rows(int S, int K, int E, int cap, int row_align) 
     return ab_round_up(kept + (int64_t)E * (row_align - 1), row_align);
 }
 
-extern "C" size_t ab_moe_plan_workspace_bytes(int S, int K, int E) {
-    (void)E;
-    return (size_t)ab_round_up((int64_t)S * K * sizeof(int32_t), 256);
+namespace {
+// plan workspace: row_local [S*K] | zeroed: histograms [4][E*K][256], tickets [8], any_select | sel [E*K] | cc [chunks][K][E][2]
+struct PlanWs { size_t hist_off, zero_bytes, sel_off, cc_off, total; };
+PlanWs plan_ws(int S, int K, int E) {
+    PlanWs p;
+    size_t o = ab_round_up((int64_t)S * K * sizeof(int32_t), 256);
+    p.hist_off = o;
+    p.zero_bytes = ab_round_up(((int64_t)4 * E * K * 256 + 16) * sizeof(int), 256);
+    o += p.zero_bytes;
+    p.sel_off = o; o += ab_round_up((int64_t)E * K * sizeof(PlanSel), 256);
+    p.cc_off = o; o += ab_round_up(ab_ceil_div(S, PLAN_CHUNK) * K * 2 * E * (int64_t)sizeof(int), 256);
+    p.total = o;
+    return p;
 }
+}  // namespace
+
+extern "C" size_t ab_moe_plan_workspace_bytes(int S, int K, int E) { return plan_ws(S, K, E).total; }
 
 extern "C" int ab_moe_plan(const int32_t* idx, const float* w, const int32_t* active, int cap, int32_t* counts,
                            int32_t* seg_off, int32_t* row_of, int32_t* tok_of_row, int32_t* slot_of_row,
@@ -767,16 +812,27 @@ extern "C" int ab_moe_plan(const int32_t* idx, const float* w, const int32_t* ac
         AB_REQUIRE(row_align > 0 && max_rows % row_align == 0 && max_rows >= ab_moe_max_rows(S, K, E, cap < S ? cap : S, row_align),
                    "moe_plan: max_rows %lld too small or not a multiple of %d", (long long)max_rows, row_align);
     }
-    AB_REQUIRE(ws && ws_bytes >= ab_moe_plan_workspace_bytes(S, K, E), "moe_plan: workspace too small");
+    const PlanWs pw = plan_ws(S, K, E);
+    AB_REQUIRE(ws && ws_bytes >= pw.total, "moe_plan: workspace too small");
+    unsigned char* w8 = (unsigned char*)ws;
     int32_t* row_local = (int32_t*)ws;
+    int* ghist = (int*)(w8 + pw.hist_off);
+    int* tickets = ghist + (size_t)4 * E * K * 256;            // [0..3] histogram passes
+    int* any_select = tickets + 8;
+    PlanSel* sel = (PlanSel*)(w8 + pw.sel_off);
+    int* cc = (int*)(w8 + pw.cc_off);
+    AB_CHECK_CUDA(cudaMemsetAsync(ghist, 0, pw.zero_bytes, stream));
     AB_CHECK_CUDA(cudaMemsetAsync(tok_of_row, 0xFF, (size_t)max_rows * sizeof(int32_t), stream));
     AB_CHECK_CUDA(cudaMemsetAsync(slot_of_row, 0xFF, (size_t)max_rows * sizeof(int32_t), stream));
-    // candidate list in shared memory: as many entries as fit (8 B each), at most S
-    int list_cap = (200 * 1024) / 8;
-    if (list_cap > S) list_cap = S;
-    const size_t plan_smem = (size_t)list_cap * sizeof(uint2);
-    AB_CHECK_CUDA(cudaFuncSetAttribute(plan_count_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan_smem));
-    plan_count_kernel<<<E, PLAN_THREADS, plan_smem, stream>>>(idx, w, active, cap, counts, row_local, S, K, list_cap);
+    const dim3 hgrid((unsigned)ab_ceil_div(S, HIST_TOKENS), K), cgrid((unsigned)ab_ceil_div(S, PLAN_CHUNK), K);
+    for (int pass = 3; pass >= 0; --pass) {
+        plan_hist_kernel<<<hgrid, PLAN_THREADS, 0, stream>>>(idx, w, active, cap, pass, ghist + (size_t)(3 - pass) * E * K * 256, sel,
+                                                             any_select, tickets + (3 - pass), counts, S, K, E);
+        AB_LAUNCH_CHECK();
+    }
+    plan_chunk_count_kernel<<<cgrid, PLAN_THREADS, 0, stream>>>(idx, w, sel, cc, S, K, E);
+    AB_LAUNCH_CHECK();
+    plan_pos_kernel<<<cgrid, PLAN_THREADS, 0, stream>>>(idx, w, sel, cc, row_local, S, K, E);
     AB_LAUNCH_CHECK();
     const int64_t want = ab_ceil_div((int64_t)S * K, 256);
     const int grid = (int)(want < ab_num_sms() * 4 ? want : ab_num_sms() * 4);

@@ -26,6 +26,28 @@ __device__ __forceinline__ void row_load(const T* row, int i, float* f) {   // v
     ab_vec16<T>::unpack(__ldg(reinterpret_cast<const uint4*>(row) + i), f);
 }
 
+// four consecutive elements: one 16-byte (fp32) or 8-byte (bf16) access
+template <typename T>
+__device__ __forceinline__ void ld4g(const T* p, float* f) {
+    if constexpr (sizeof(T) == 4) {
+        const float4 q = __ldg(reinterpret_cast<const float4*>(p));
+        f[0] = q.x; f[1] = q.y; f[2] = q.z; f[3] = q.w;
+    } else {
+        const uint2 r = __ldg(reinterpret_cast<const uint2*>(p));
+        f[0] = __uint_as_float(r.x << 16); f[1] = __uint_as_float(r.x & 0xffff0000u);
+        f[2] = __uint_as_float(r.y << 16); f[3] = __uint_as_float(r.y & 0xffff0000u);
+    }
+}
+template <typename T>
+__device__ __forceinline__ void ab_st4(T* p, const float* o) {
+    if constexpr (sizeof(T) == 4) {
+        *reinterpret_cast<float4*>(p) = make_float4(o[0], o[1], o[2], o[3]);
+    } else {
+        __nv_bfloat162 lo = __floats2bfloat162_rn(o[0], o[1]), hi = __floats2bfloat162_rn(o[2], o[3]);
+        *reinterpret_cast<uint2*>(p) = make_uint2(*reinterpret_cast<uint32_t*>(&lo), *reinterpret_cast<uint32_t*>(&hi));
+    }
+}
+
 // softmax / top-K / weights on lanes (lane e < E holds logit e).  Returns the gate in g; lane k < K ends up holding
 // slot k's expert id and probability (my_idx, my_p) -- no per-thread arrays, so nothing spills to local memory.
 __device__ __forceinline__ void select_topk(float logit, int lane, int E, int K, float& g, float& lse, int& my_idx, float& my_p,
@@ -234,7 +256,16 @@ __device__ __forceinline__ float reduce_dots_to_lane(float (&dot)[EM], int lane,
 }
 
 template <typename T, int EM, int NV>
-__global__ void __launch_bounds__(WARPS * 32, (NV * ab_vec16<T>::N <= 24 && EM <= 8) ? 4 : 1) router_fwd_reg_kernel(const T* __restrict__ x, const float* __restrict__ ln_w,
+#ifndef FWD_MINB
+#define FWD_MINB 2
+#endif
+#ifndef FWD_REGPF
+#define FWD_REGPF 1
+#endif
+#ifndef FWD_PERSIST
+#define FWD_PERSIST 1
+#endif
+__global__ void __launch_bounds__(WARPS * 32, (NV * ab_vec16<T>::N <= 24 && EM <= 8) ? FWD_MINB : 1) router_fwd_reg_kernel(const T* __restrict__ x, const float* __restrict__ ln_w,
                                                                     const float* __restrict__ ln_b, float eps,
                                                                     const float* __restrict__ Wr, const float* __restrict__ br,
                                                                     const float* __restrict__ noise,
@@ -269,20 +300,46 @@ __global__ void __launch_bounds__(WARPS * 32, (NV * ab_vec16<T>::N <= 24 && EM <
     const int nvec = Dm / V;
     const float inv_dm = 1.0f / (float)Dm;
     float a_g = 0.f, a_cnt = 0.f, a_l2 = 0.f;
-    for (int s = blockIdx.x * WARPS + warp; s < S; s += gridDim.x * WARPS) {
+    // the warp's next row is loaded while the current one is reduced: its loads are in flight during the dependent chain
+    // of reductions, dot products and top-K of this row.  Rows of more than 64 values per lane would not fit twice.
+    constexpr bool PF = FWD_REGPF && NV * V <= 64;
+    float fn[NV][V];
+    auto load_row = [&](int s) {
         const T* row = x + (size_t)s * Dm;
-        float f[NV][V];
-        float sum = 0.f;
 #pragma unroll
         for (int i = 0; i < NV; ++i) {
             const int iv = i * 32 + lane;
-            if (iv < nvec) {
-                row_load<T>(row, iv, f[i]);
-#pragma unroll
-                for (int v = 0; v < V; ++v) sum += f[i][v];
+            if (s < S && iv < nvec) {
+                row_load<T>(row, iv, fn[i]);
             } else {
 #pragma unroll
-                for (int v = 0; v < V; ++v) f[i][v] = 0.f;
+                for (int v = 0; v < V; ++v) fn[i][v] = 0.f;
+            }
+        }
+    };
+    const int stride = gridDim.x * WARPS;
+    if constexpr (PF) load_row(blockIdx.x * WARPS + warp);
+    for (int s = blockIdx.x * WARPS + warp; s < S; s += stride) {
+        if constexpr (!PF) {
+            load_row(s);
+            // the warp's next row into L2 while this one is reduced (no registers held)
+            const char* nx = reinterpret_cast<const char*>(x + (size_t)(s + stride) * Dm);
+            if (s + stride < S)
+                for (int o = lane * 128; o < Dm * (int)sizeof(T); o += 32 * 128) asm volatile("prefetch.global.L2 [%0];" ::"l"(nx + o));
+        }
+        float f[NV][V];
+#pragma unroll
+        for (int i = 0; i < NV; ++i) {
+#pragma unroll
+            for (int v = 0; v < V; ++v) f[i][v] = fn[i][v];
+        }
+        if constexpr (PF) load_row(s + stride);
+        float sum = 0.f;
+#pragma unroll
+        for (int i = 0; i < NV; ++i) {
+            if (i * 32 + lane < nvec) {
+#pragma unroll
+                for (int v = 0; v < V; ++v) sum += f[i][v];
             }
         }
         const float mean = ab_warp_sum(sum) * inv_dm;
@@ -387,9 +444,73 @@ __global__ void __launch_bounds__(WARPS * 32) topk_from_logits_kernel(const floa
 }
 
 // ---------------------------------------------------------------------------------------------
-// backward, kernel B: per token d logits and dx
+// backward: per token d logits and dx
 // part layout per CTA: [2E] = sum dlogit[e] (-> dbr), sum dlogit[e]*noise[s,e] (-> dnoise_scale)
 // ---------------------------------------------------------------------------------------------
+// The per-token scalars of the backward (warp per token): lane e < E gets d logit e, lane k < K the row of slot k (-1 if
+// dropped); every lane gets mean, rstd and the LayerNorm constants m1 = mean_d(dxhat), m2 = mean_d(dxhat * xhat).
+// a_db / a_dn accumulate the lane's d logit and d logit * noise.
+__device__ __forceinline__ void router_token_grad(int s, int lane, int E, int K, int Dm, const float* GS, const float* cvec,
+                                                  const float* __restrict__ stats, const float* __restrict__ gates,
+                                                  const int32_t* __restrict__ idx, const float* __restrict__ probs,
+                                                  const float* __restrict__ lse, const float* __restrict__ lclean,
+                                                  const float* __restrict__ noise, const float* __restrict__ f, float g_lb,
+                                                  float g_rz, const float* __restrict__ dw_row, const int32_t* __restrict__ row_of,
+                                                  int& my_r, float& dl, float& mean, float& rstd, float& m1, float& m2,
+                                                  float& a_db, float& a_dn) {
+    // loads that do not depend on the slot rows first: one memory latency for all of them
+    const float g_in = lane < E ? gates[(size_t)s * E + lane] : 0.f;
+    const float lse_s = lse[s];
+    const float lc_in = lane < E ? lclean[(size_t)s * E + lane] : 0.f;
+    const float nz_in = noise != nullptr && lane < E ? noise[(size_t)s * E + lane] : 0.f;
+    const float f_in = lane < E ? f[lane] : 0.f;
+    mean = stats[2 * (size_t)s]; rstd = stats[2 * (size_t)s + 1];
+    // ---- d weights -> d probs (lane k < K holds slot k)
+    int my_i = 0;
+    float my_dw = 0.f, my_pk = 0.f;
+    my_r = -1;
+    if (lane < K) {
+        my_r = row_of[(size_t)s * K + lane];
+        my_i = idx[(size_t)s * K + lane];
+        my_pk = probs[(size_t)s * K + lane];
+        my_dw = my_r >= 0 ? dw_row[my_r] : 0.f;
+    }
+    float den = 0.f;
+    for (int k = 0; k < K; ++k) den += __shfl_sync(0xffffffffu, my_pk, k);    // slot order, as in the forward
+    den += 1e-6f;
+    const float dot = ab_warp_sum(my_dw * my_pk);
+    const float inv = 1.f / den;
+    const float my_dp = my_dw * inv - dot * inv * inv;       // d prob of slot `lane`
+    float dgate = 0.f, g = 0.f;
+    for (int k = 0; k < K; ++k) {
+        const int ik = __shfl_sync(0xffffffffu, my_i, k);
+        const float dpk = __shfl_sync(0xffffffffu, my_dp, k);
+        if (lane == ik) dgate += dpk;
+    }
+    if (lane < E) {
+        g = g_in;
+        dgate = fmaf(g_lb, f_in, dgate);
+    } else {
+        dgate = 0.f;
+    }
+    const float gd = ab_warp_sum(g * dgate);
+    dl = 0.f;
+    if (lane < E) {
+        dl = g * (dgate - gd) + g_rz * 2.f * lse_s * g;
+        a_db += dl;
+        if (noise) a_dn = fmaf(dl, nz_in, a_dn);
+    }
+    // ---- LayerNorm backward constants
+    float t1 = 0.f, t2 = 0.f;
+    if (lane < E) {
+        t1 = dl * GS[lane];
+        t2 = dl * (lc_in - cvec[lane]);    // sum_d G[e,d]*xhat[d]
+    }
+    m1 = ab_warp_sum(t1) / (float)Dm;
+    m2 = ab_warp_sum(t2) / (float)Dm;
+}
+
+// Row kernel (warp per token) for the shapes the one-pass kernels below do not take; router_q_kernel then forms Q.
 template <typename T, int EM>
 __global__ void __launch_bounds__(WARPS * 32) router_bwd_kernel(const T* __restrict__ x, const float* __restrict__ stats,
                                                                 const float* __restrict__ ln_w, const float* __restrict__ ln_b,
@@ -426,50 +547,11 @@ __global__ void __launch_bounds__(WARPS * 32) router_bwd_kernel(const T* __restr
     const int nvec = Dm / V;
     float a_db = 0.f, a_dn = 0.f;
     for (int s = blockIdx.x * WARPS + warp; s < S; s += gridDim.x * WARPS) {
-        // ---- d weights -> d probs (lane k < K holds slot k)
-        int my_r = -1, my_i = 0;
-        float my_dw = 0.f, my_pk = 0.f;
-        if (lane < K) {
-            my_r = row_of[(size_t)s * K + lane];
-            my_i = idx[(size_t)s * K + lane];
-            my_pk = probs[(size_t)s * K + lane];
-            my_dw = my_r >= 0 ? dw_row[my_r] : 0.f;
-        }
-        float den = 0.f;
-        for (int k = 0; k < K; ++k) den += __shfl_sync(0xffffffffu, my_pk, k);    // slot order, as in the forward
-        den += 1e-6f;
-        const float dot = ab_warp_sum(my_dw * my_pk);
-        const float inv = 1.f / den;
-        const float my_dp = my_dw * inv - dot * inv * inv;       // d prob of slot `lane`
-        float dgate = 0.f, g = 0.f;
-        for (int k = 0; k < K; ++k) {
-            const int ik = __shfl_sync(0xffffffffu, my_i, k);
-            const float dpk = __shfl_sync(0xffffffffu, my_dp, k);
-            if (lane == ik) dgate += dpk;
-        }
-        if (lane < E) {
-            g = gates[(size_t)s * E + lane];
-            dgate = fmaf(g_lb, f[lane], dgate);
-        } else {
-            dgate = 0.f;
-        }
-        const float gd = ab_warp_sum(g * dgate);
-        float dl = 0.f;
-        if (lane < E) {
-            dl = g * (dgate - gd) + g_rz * 2.f * lse[s] * g;
-            dlogits[(size_t)s * E + lane] = dl;
-            a_db += dl;
-            if (noise) a_dn = fmaf(dl, noise[(size_t)s * E + lane], a_dn);
-        }
-        // ---- LayerNorm backward constants:  m1 = mean_d(dxhat), m2 = mean_d(dxhat * xhat)
-        const float mean = stats[2 * (size_t)s], rstd = stats[2 * (size_t)s + 1];
-        float t1 = 0.f, t2 = 0.f;
-        if (lane < E) {
-            t1 = dl * GS[lane];
-            t2 = dl * (lclean[(size_t)s * E + lane] - cvec[lane]);    // sum_d G[e,d]*xhat[d]
-        }
-        const float m1 = ab_warp_sum(t1) / (float)Dm;
-        const float m2 = ab_warp_sum(t2) / (float)Dm;
+        int my_r;
+        float dl, mean, rstd, m1, m2;
+        router_token_grad(s, lane, E, K, Dm, GS, cvec, stats, gates, idx, probs, lse, lclean, noise, f, g_lb, g_rz, dw_row, row_of,
+                          my_r, dl, mean, rstd, m1, m2, a_db, a_dn);
+        if (lane < E) dlogits[(size_t)s * E + lane] = dl;
         float dle[EM];
 #pragma unroll
         for (int e = 0; e < EM; ++e) dle[e] = __shfl_sync(0xffffffffu, dl, e);
@@ -571,9 +653,205 @@ __global__ void __launch_bounds__(256) router_q_kernel(const T* __restrict__ x, 
         if (e < E) qpart[((size_t)blockIdx.y * E + e) * Dm + d] = acc[e];
 }
 
-// kernel D: reduce Q partials and derive all router parameter grads.  block = (32 columns, E experts)
+// Backward for E <= 8 and hidden sizes up to 1024 in one pass over x, split in two kernels so that neither waits on the
+// other's latency chain.  router_bwd_tok_kernel (warp per token, the whole grid): the per-token scalars of
+// router_token_grad -> tsc[s] = {d logits [8], mean, rstd, m1, m2}, and the per-CTA sums for dbr / dnoise_scale.
+constexpr int TSC = 12;                      // floats per token in tsc
+constexpr int TOK_CTAS_PER_SM = 6;           // 48 warps per SM on the token kernel's latency-bound chains
+constexpr int FUSED_EM = 8;
+__global__ void __launch_bounds__(WARPS * 32, TOK_CTAS_PER_SM) router_bwd_tok_kernel(const float* __restrict__ stats, const float* __restrict__ ln_w,
+                                                                    const float* __restrict__ ln_b, const float* __restrict__ Wr,
+                                                                    const float* __restrict__ br, const float* __restrict__ gates,
+                                                                    const int32_t* __restrict__ idx, const float* __restrict__ probs,
+                                                                    const float* __restrict__ lse, const float* __restrict__ lclean,
+                                                                    const float* __restrict__ noise, const float* __restrict__ f,
+                                                                    const float* __restrict__ scal, const float* __restrict__ dw_row,
+                                                                    const int32_t* __restrict__ row_of, float* __restrict__ tsc,
+                                                                    float* __restrict__ part, int S, int Dm, int E, int K) {
+    __shared__ float GS[32], cvec[32], red[WARPS][2 * FUSED_EM];
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    for (int e = warp; e < E; e += WARPS) {
+        float a1 = 0.f, a2 = 0.f;
+        for (int d = lane; d < Dm; d += 32) {
+            a1 = fmaf(ln_w[d], Wr[(size_t)e * Dm + d], a1);
+            a2 = fmaf(ln_b[d], Wr[(size_t)e * Dm + d], a2);
+        }
+        a1 = ab_warp_sum(a1); a2 = ab_warp_sum(a2);
+        if (lane == 0) { GS[e] = a1; cvec[e] = a2 + br[e]; }
+    }
+    __syncthreads();
+    const float g_lb = scal[0], g_rz = scal[1];
+    float a_db = 0.f, a_dn = 0.f;
+    for (int s = blockIdx.x * WARPS + warp; s < S; s += gridDim.x * WARPS) {
+        int my_r;
+        float dl, mean, rstd, m1, m2;
+        router_token_grad(s, lane, E, K, Dm, GS, cvec, stats, gates, idx, probs, lse, lclean, noise, f, g_lb, g_rz, dw_row, row_of,
+                          my_r, dl, mean, rstd, m1, m2, a_db, a_dn);
+        float v = dl;                                // lanes < 8: d logit (0 for lanes >= E)
+        if (lane == 8) v = mean;
+        if (lane == 9) v = rstd;
+        if (lane == 10) v = m1;
+        if (lane == 11) v = m2;
+        if (lane < TSC) tsc[(size_t)s * TSC + lane] = v;
+    }
+    const int NA = 2 * E;
+    if (lane < E) { red[warp][lane] = a_db; red[warp][E + lane] = a_dn; }
+    __syncthreads();
+    if (tid < NA) {
+        float s2 = 0.f;
+        for (int wv = 0; wv < WARPS; ++wv) s2 += red[wv][tid];
+        part[(size_t)blockIdx.x * NA + tid] = s2;
+    }
+}
+
+// router_bwd_col_kernel: a persistent CTA takes tiles of BT tokens; thread c owns the columns [4c, 4c+4) of every row of
+// the tile, forms dx there and accumulates Q[e,d] = sum_s dlogits[s,e] * xhat[s,d] in registers over all its tiles.  The
+// CTA's Q partial is written once at the end; router_param_kernel adds the partials in CTA order.  dx is computed with
+// the same operations in the same order as in router_bwd_kernel.  The next tile's scalars and slot rows are copied to
+// shared memory asynchronously while the current tile streams.
+constexpr int BT = 32;
+constexpr int FUSED_MAX_THREADS = 256;
+constexpr int FUSED_MAX_REGS = 144;          // no spills; two CTAs of 192 threads (hidden 704) per SM
+template <typename T, int KM>
+__global__ void __maxnreg__(FUSED_MAX_REGS) router_bwd_col_kernel(const T* __restrict__ x, const float* __restrict__ ln_w,
+                                                                  const float* __restrict__ Wr, const float* __restrict__ tsc,
+                                                                  const float* __restrict__ dxrow, const int32_t* __restrict__ row_of,
+                                                                  T* __restrict__ dx, float* __restrict__ qpart, int S, int Dm,
+                                                                  int E, int K) {
+    constexpr int EM = FUSED_EM;
+    constexpr int U = KM <= 2 ? 4 : 1;       // tokens whose loads are issued together
+    constexpr int NSC = BT * TSC, NROW = BT * KM;
+    extern __shared__ float sm[];
+    float* Wsm = sm;                         // [E][Dm] raw router weight
+    float* stile = Wsm + (size_t)E * Dm;     // [2][BT][TSC] scalars of the tile (double buffer)
+    int* srow = reinterpret_cast<int*>(stile + 2 * NSC);    // [2][BT][KM] rows of the slots, -1 if dropped
+    const int tid = threadIdx.x;
+    for (int i = tid; i < E * Dm; i += blockDim.x) Wsm[i] = Wr[i];
+    const int d = 4 * tid;
+    const bool has_col = d < Dm;
+    float gg[4] = {0.f, 0.f, 0.f, 0.f};
+    if (has_col) {
+        const float4 gq = __ldg(reinterpret_cast<const float4*>(ln_w + d));
+        gg[0] = gq.x; gg[1] = gq.y; gg[2] = gq.z; gg[3] = gq.w;
+    }
+    // one tile's scalars and rows into buffer `buf` by asynchronous copies (no registers held while they are in flight);
+    // complete after cp.async.wait_all
+    auto fetch = [&](int s0, int buf) {
+        const int nt = s0 < S ? min(BT, S - s0) : 0;
+        for (int i = tid; i < nt * TSC; i += blockDim.x) {
+            const unsigned dst = (unsigned)__cvta_generic_to_shared(stile + buf * NSC + i);
+            asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(dst), "l"(tsc + (size_t)s0 * TSC + i));
+        }
+        for (int i = tid; i < nt * KM; i += blockDim.x) {
+            const int j = i / KM, k = i % KM;
+            if (k < K) {
+                const unsigned dst = (unsigned)__cvta_generic_to_shared(srow + buf * NROW + i);
+                asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(dst), "l"(row_of + (size_t)(s0 + j) * K + k));
+            } else {
+                srow[buf * NROW + i] = -1;
+            }
+        }
+    };
+    float q[EM][4];
+#pragma unroll
+    for (int e = 0; e < EM; ++e) { q[e][0] = q[e][1] = q[e][2] = q[e][3] = 0.f; }
+    const int step = gridDim.x * BT;
+    fetch(blockIdx.x * BT, 0);
+    asm volatile("cp.async.wait_all;" ::: "memory");
+    __syncthreads();
+    int buf = 0;
+    for (int s0 = blockIdx.x * BT; s0 < S; s0 += step, buf ^= 1) {
+        const int nt = min(BT, S - s0);
+        fetch(s0 + step, buf ^ 1);
+        const float* sc = stile + buf * NSC;
+        const int* rw = srow + buf * NROW;
+        if (has_col) {
+            for (int j0 = 0; j0 < nt; j0 += U) {
+                // the next batch's x and dxrow lines into L2 (no registers held): its loads then wait on L2, not HBM
+#pragma unroll
+                for (int u = 0; u < U; ++u) {
+                    const int j = j0 + U + u;
+                    if (j < nt && (tid & 7) == 0) {          // one thread per 128-byte line of fp32 rows
+                        asm volatile("prefetch.global.L2 [%0];" ::"l"(x + (size_t)(s0 + j) * Dm + d));
+#pragma unroll
+                        for (int k = 0; k < KM; ++k) {
+                            const int r = rw[j * KM + k];
+                            if (r >= 0) asm volatile("prefetch.global.L2 [%0];" ::"l"(dxrow + (size_t)r * Dm + d));
+                        }
+                    }
+                }
+                float xv[U][4], er[U][KM][4];
+#pragma unroll
+                for (int u = 0; u < U; ++u) {
+                    const int j = j0 + u;
+#pragma unroll
+                    for (int k = 0; k < KM; ++k) er[u][k][0] = er[u][k][1] = er[u][k][2] = er[u][k][3] = 0.f;
+                    xv[u][0] = xv[u][1] = xv[u][2] = xv[u][3] = 0.f;
+                    if (j < nt) {
+                        ld4g<T>(x + (size_t)(s0 + j) * Dm + d, xv[u]);
+#pragma unroll
+                        for (int k = 0; k < KM; ++k) {
+                            const int r = rw[j * KM + k];
+                            if (r >= 0) ld4g<float>(dxrow + (size_t)r * Dm + d, er[u][k]);
+                        }
+                    }
+                }
+#pragma unroll
+                for (int u = 0; u < U; ++u) {
+                    const int j = j0 + u;
+                    if (j >= nt) break;
+                    const float* t = sc + j * TSC;
+                    const float mean = t[8], rstd = t[9], m1 = t[10], m2 = t[11];
+                    float dle[EM];
+#pragma unroll
+                    for (int e = 0; e < EM; ++e) dle[e] = t[e];
+                    float dxn[4] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll
+                    for (int e = 0; e < EM; ++e) {
+                        if (e < E) {
+                            const float4 wq = *reinterpret_cast<const float4*>(Wsm + (size_t)e * Dm + d);
+                            dxn[0] = fmaf(dle[e], wq.x, dxn[0]); dxn[1] = fmaf(dle[e], wq.y, dxn[1]);
+                            dxn[2] = fmaf(dle[e], wq.z, dxn[2]); dxn[3] = fmaf(dle[e], wq.w, dxn[3]);
+                        }
+                    }
+                    float o[4], xh[4];
+#pragma unroll
+                    for (int v = 0; v < 4; ++v) {
+                        xh[v] = (xv[u][v] - mean) * rstd;
+                        o[v] = rstd * (dxn[v] * gg[v] - m1 - xh[v] * m2);
+                    }
+#pragma unroll
+                    for (int k = 0; k < KM; ++k) {
+                        if (rw[j * KM + k] >= 0) {
+#pragma unroll
+                            for (int v = 0; v < 4; ++v) o[v] += er[u][k][v];
+                        }
+                    }
+                    ab_st4<T>(dx + (size_t)(s0 + j) * Dm + d, o);
+#pragma unroll
+                    for (int e = 0; e < EM; ++e) {
+#pragma unroll
+                        for (int v = 0; v < 4; ++v) q[e][v] = fmaf(dle[e], xh[v], q[e][v]);
+                    }
+                }
+            }
+        }
+        asm volatile("cp.async.wait_all;" ::: "memory");
+        __syncthreads();
+    }
+    if (has_col) {
+#pragma unroll
+        for (int e = 0; e < EM; ++e)
+            if (e < E) *reinterpret_cast<float4*>(qpart + ((size_t)blockIdx.x * E + e) * Dm + d) = make_float4(q[e][0], q[e][1], q[e][2], q[e][3]);
+    }
+}
+
+// kernel D: reduce Q partials and derive all router parameter grads.  block = (32 columns, E experts, G row groups)
 //   dbr[e] = sum dlogits;  dWr[e,d] = ln_w[d]*Q[e,d] + ln_b[d]*dbr[e]
 //   dln_w[d] = sum_e Wr[e,d]*Q[e,d];  dln_b[d] = sum_e Wr[e,d]*dbr[e]
+// Group g adds the partial rows g, g+G, ... in order, then the G group sums are added in group order (fixed order ->
+// deterministic); the groups put G times as many loads in flight.
+int param_groups(int E) { const int g = 1024 / (32 * E); return g < 1 ? 1 : (g > 4 ? 4 : g); }
 __global__ void router_param_kernel(const float* __restrict__ qpart, int nqb, const float* __restrict__ part, int nparts,
                                     const float* __restrict__ ln_w, const float* __restrict__ ln_b, const float* __restrict__ Wr,
                                     float* __restrict__ dWr, float* __restrict__ dbr, float* __restrict__ dln_w,
@@ -581,25 +859,26 @@ __global__ void router_param_kernel(const float* __restrict__ qpart, int nqb, co
     __shared__ float sdb[64];
     __shared__ float sgw[32][33], sgb[32][33];
     __shared__ float spart[16][64];
-    const int tx = threadIdx.x, e = threadIdx.y;
-    const int tid = e * 32 + tx;
-    const int nthr = 32 * E;
+    __shared__ float sq[32][33];             // [group * E + e][column]
+    const int tx = threadIdx.x, e = threadIdx.y, grp = threadIdx.z, G = blockDim.z;
+    const int tid = (grp * E + e) * 32 + tx;
+    const int nthr = 32 * E * G;
     // column sums of the per-CTA partials: up to 16 thread groups add interleaved rows, then one thread per column adds
     // the groups in index order (fixed order -> deterministic)
     {
         const int ncol = 2 * E;
         const int ngrp = min(16, nthr / ncol);
-        const int col = tid % ncol, grp = tid / ncol;
-        if (grp < ngrp) {
+        const int col = tid % ncol, pg = tid / ncol;
+        if (pg < ngrp) {
             float s = 0.f;
-            for (int r0 = grp; r0 < nparts; r0 += ngrp * 4) {
+            for (int r0 = pg; r0 < nparts; r0 += ngrp * 4) {
                 float v[4];
 #pragma unroll
                 for (int u = 0; u < 4; ++u) v[u] = r0 + u * ngrp < nparts ? part[(size_t)(r0 + u * ngrp) * ncol + col] : 0.f;
 #pragma unroll
                 for (int u = 0; u < 4; ++u) s += v[u];
             }
-            spart[grp][col] = s;
+            spart[pg][col] = s;
         }
         __syncthreads();
         if (tid < ncol) {
@@ -612,27 +891,36 @@ __global__ void router_param_kernel(const float* __restrict__ qpart, int nqb, co
             }
         }
     }
-    __syncthreads();
     const int d = blockIdx.x * 32 + tx;
-    float gw = 0.f, gb = 0.f;
-    if (d < Dm) {
+    {
         float q = 0.f;
-        for (int r0 = 0; r0 < nqb; r0 += 8) {
-            float qv[8];
+        if (d < Dm) {
+            for (int r0 = grp; r0 < nqb; r0 += 8 * G) {
+                float qv[8];
 #pragma unroll
-            for (int u = 0; u < 8; ++u) qv[u] = r0 + u < nqb ? qpart[((size_t)(r0 + u) * E + e) * Dm + d] : 0.f;
+                for (int u = 0; u < 8; ++u) qv[u] = r0 + u * G < nqb ? qpart[((size_t)(r0 + u * G) * E + e) * Dm + d] : 0.f;
 #pragma unroll
-            for (int u = 0; u < 8; ++u) q += qv[u];
+                for (int u = 0; u < 8; ++u) q += qv[u];
+            }
         }
-        const float wv = Wr[(size_t)e * Dm + d];
-        dWr[(size_t)e * Dm + d] = fmaf(ln_w[d], q, ln_b[d] * sdb[e]);
-        gw = wv * q;
-        gb = wv * sdb[e];
+        sq[grp * E + e][tx] = q;
     }
-    sgw[e][tx] = gw;
-    sgb[e][tx] = gb;
     __syncthreads();
-    if (e == 0 && d < Dm) {
+    if (grp == 0) {
+        float gw = 0.f, gb = 0.f;
+        if (d < Dm) {
+            float q = 0.f;
+            for (int g2 = 0; g2 < G; ++g2) q += sq[g2 * E + e][tx];
+            const float wv = Wr[(size_t)e * Dm + d];
+            dWr[(size_t)e * Dm + d] = fmaf(ln_w[d], q, ln_b[d] * sdb[e]);
+            gw = wv * q;
+            gb = wv * sdb[e];
+        }
+        sgw[e][tx] = gw;
+        sgb[e][tx] = gb;
+    }
+    __syncthreads();
+    if (grp == 0 && e == 0 && d < Dm) {
         float a = 0.f, b = 0.f;
         for (int i = 0; i < E; ++i) { a += sgw[i][tx]; b += sgb[i][tx]; }
         dln_w[d] = a;
@@ -654,14 +942,24 @@ FwdWs fwd_ws(int S, int E) {
     w.total = ab_round_up((int64_t)w.grid * (2 * E + 1) * sizeof(float), 256);
     return w;
 }
-struct BwdWs { size_t part_off, dl_off, q_off, total; int grid, nqb; };
+// the one-pass backward takes E <= 8 and hidden sizes up to 4 * FUSED_MAX_THREADS; its column kernel runs at most
+// MAX_FUSED_PER_SM CTAs per SM
+constexpr int MAX_FUSED_PER_SM = 4;
+// the token kernel in one wave of TOK_CTAS_PER_SM CTAs per SM
+int tok_grid(int S) {
+    const int want = (int)ab_ceil_div(S, WARPS);
+    const int cap = ab_num_sms() * TOK_CTAS_PER_SM;
+    return want < cap ? want : cap;
+}
+bool bwd_fused(int Dm, int E) { return E <= FUSED_EM && Dm % 4 == 0 && Dm / 4 <= FUSED_MAX_THREADS; }
+struct BwdWs { size_t part_off, dl_off, q_off, total; int nqb; };
 BwdWs bwd_ws(int S, int Dm, int E) {
     BwdWs w;
-    w.grid = router_grid(S);
-    w.nqb = (int)ab_ceil_div(S, qb_for(em_for(E)));
+    const bool fused = bwd_fused(Dm, E);
+    w.nqb = fused ? ab_num_sms() * MAX_FUSED_PER_SM : (int)ab_ceil_div(S, qb_for(em_for(E)));
     size_t o = 0;
-    w.part_off = o; o += ab_round_up((int64_t)w.grid * 2 * E * sizeof(float), 256);
-    w.dl_off = o; o += ab_round_up((int64_t)S * E * sizeof(float), 256);
+    w.part_off = o; o += ab_round_up((int64_t)(fused ? tok_grid(S) : router_grid(S)) * 2 * E * sizeof(float), 256);
+    w.dl_off = o; o += ab_round_up((int64_t)S * (fused ? TSC : E) * sizeof(float), 256);     // tsc, or the d logits
     w.q_off = o; o += ab_round_up((int64_t)w.nqb * E * Dm * sizeof(float), 256);
     w.total = o;
     return w;
@@ -694,12 +992,17 @@ extern "C" int ab_moe_router_fwd(const void* x, const float* ln_w, const float* 
     float* part = (float*)ws;
     const int V = dtype == AB_F32 ? 4 : 8;
     const int nv = (int)ab_ceil_div(Dm, 32 * V);          // 16-byte vectors of the row per lane
+    int grid = wl.grid;
 #define AB_ROUTER_LAUNCH(KERNEL)                                                                                        \
     {                                                                                                                    \
         auto k = KERNEL;                                                                                                 \
         AB_CHECK_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));                 \
-        k<<<wl.grid, WARPS * 32, smem, stream>>>((const TT*)x, ln_w, ln_b, eps, Wr, br, noise, noise_scale, lclean,     \
-                                                 logits, gates, idx, probs, w, lse, stats_out, part, S, Dm, E, K, quant); \
+        int occ = 4;                                                                                                     \
+        if (FWD_PERSIST) AB_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k, WARPS * 32, smem));       \
+        occ = occ < 1 ? 1 : (occ > 4 ? 4 : occ);                                                                        \
+        grid = wl.grid < ab_num_sms() * occ ? wl.grid : ab_num_sms() * occ;                                              \
+        k<<<grid, WARPS * 32, smem, stream>>>((const TT*)x, ln_w, ln_b, eps, Wr, br, noise, noise_scale, lclean,         \
+                                              logits, gates, idx, probs, w, lse, stats_out, part, S, Dm, E, K, quant);    \
     }
     // the row-in-registers kernel whenever the row fits (hidden size <= 2048 fp32 / 4096 bf16), the streaming one otherwise
 #define AB_ROUTER_FWD(TT_, EMV)                                                                                         \
@@ -719,7 +1022,7 @@ extern "C" int ab_moe_router_fwd(const void* x, const float* ln_w, const float* 
 #undef AB_ROUTER_LAUNCH
 #undef AB_ROUTER_FWD
     AB_LAUNCH_CHECK();
-    reduce_rows_kernel<<<(unsigned)ab_ceil_div(2 * E + 1, 4), 128, 0, stream>>>(part, wl.grid, 2 * E + 1, aux);
+    reduce_rows_kernel<<<(unsigned)ab_ceil_div(2 * E + 1, 4), 128, 0, stream>>>(part, grid, 2 * E + 1, aux);
     AB_LAUNCH_CHECK();
     return AB_OK;
 }
@@ -748,27 +1051,56 @@ extern "C" int ab_moe_router_bwd(const void* x, const float* stats, const float*
     float* part = (float*)(w8 + wl.part_off);
     float* dl = (float*)(w8 + wl.dl_off);
     float* qpart = (float*)(w8 + wl.q_off);
-    const size_t smem = ((size_t)E * Dm + Dm + 64 + WARPS * 2 * E) * sizeof(float);
-    dim3 qgrid((unsigned)ab_ceil_div(Dm, 256), wl.nqb);
+    int nqb = wl.nqb, nparts = router_grid(S);
+    if (bwd_fused(Dm, E)) {
+        nparts = tok_grid(S);
+        router_bwd_tok_kernel<<<nparts, WARPS * 32, 0, stream>>>(stats, ln_w, ln_b, Wr, br, gates, idx, probs, lse, lclean, noise, f,
+                                                                 scal, dw_row, row_of, dl, part, S, Dm, E, K);
+        AB_LAUNCH_CHECK();
+        const int threads = (int)ab_round_up(Dm / 4 > 64 ? Dm / 4 : 64, 32);
+        const size_t smem = ((size_t)E * Dm + 2 * BT * TSC + 2 * BT * MAX_K) * sizeof(float);
+#define AB_ROUTER_BWD_COL(TT, KMV)                                                                                      \
+    {                                                                                                                    \
+        auto k = router_bwd_col_kernel<TT, KMV>;                                                                         \
+        AB_CHECK_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));                 \
+        int occ = 0;                                                                                                     \
+        AB_CHECK_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k, threads, smem));                           \
+        occ = occ < 1 ? 1 : (occ > MAX_FUSED_PER_SM ? MAX_FUSED_PER_SM : occ);                                          \
+        const int64_t want = ab_ceil_div(S, BT);                                                                         \
+        nqb = (int)(want < (int64_t)ab_num_sms() * occ ? want : (int64_t)ab_num_sms() * occ);                            \
+        k<<<nqb, threads, smem, stream>>>((const TT*)x, ln_w, Wr, dl, dxrow, row_of, (TT*)dx, qpart, S, Dm, E, K);        \
+    }
+        if (dtype == AB_F32) {
+            if (K <= 2) AB_ROUTER_BWD_COL(float, 2) else AB_ROUTER_BWD_COL(float, MAX_K)
+        } else {
+            if (K <= 2) AB_ROUTER_BWD_COL(__nv_bfloat16, 2) else AB_ROUTER_BWD_COL(__nv_bfloat16, MAX_K)
+        }
+#undef AB_ROUTER_BWD_COL
+        AB_LAUNCH_CHECK();
+    } else {
+        const size_t smem = ((size_t)E * Dm + Dm + 64 + WARPS * 2 * E) * sizeof(float);
+        dim3 qgrid((unsigned)ab_ceil_div(Dm, 256), nqb);
 #define AB_ROUTER_BWD(TT, EMV)                                                                                          \
     {                                                                                                                    \
         auto k = router_bwd_kernel<TT, EMV>;                                                                             \
         AB_CHECK_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));                 \
-        k<<<wl.grid, WARPS * 32, smem, stream>>>((const TT*)x, stats, ln_w, ln_b, Wr, br, gates, idx, probs, lse,       \
-                                                 lclean, noise, f, scal, dw_row, dxrow, row_of, (TT*)dx, dl, part, S,   \
-                                                 Dm, E, K);                                                              \
+        k<<<nparts, WARPS * 32, smem, stream>>>((const TT*)x, stats, ln_w, ln_b, Wr, br, gates, idx, probs, lse,        \
+                                                lclean, noise, f, scal, dw_row, dxrow, row_of, (TT*)dx, dl, part, S,    \
+                                                Dm, E, K);                                                               \
         AB_LAUNCH_CHECK();                                                                                               \
         router_q_kernel<TT, EMV><<<qgrid, 256, 0, stream>>>((const TT*)x, stats, dl, qpart, S, Dm, E);                  \
     }
-    if (dtype == AB_F32) {
-        if (E <= 8) AB_ROUTER_BWD(float, 8) else if (E <= 16) AB_ROUTER_BWD(float, 16) else AB_ROUTER_BWD(float, 32)
-    } else {
-        if (E <= 8) AB_ROUTER_BWD(__nv_bfloat16, 8) else if (E <= 16) AB_ROUTER_BWD(__nv_bfloat16, 16) else AB_ROUTER_BWD(__nv_bfloat16, 32)
-    }
+        if (dtype == AB_F32) {
+            if (E <= 8) AB_ROUTER_BWD(float, 8) else if (E <= 16) AB_ROUTER_BWD(float, 16) else AB_ROUTER_BWD(float, 32)
+        } else {
+            if (E <= 8) AB_ROUTER_BWD(__nv_bfloat16, 8) else if (E <= 16) AB_ROUTER_BWD(__nv_bfloat16, 16) else AB_ROUTER_BWD(__nv_bfloat16, 32)
+        }
 #undef AB_ROUTER_BWD
-    AB_LAUNCH_CHECK();
-    router_param_kernel<<<(unsigned)ab_ceil_div(Dm, 32), dim3(32, E), 0, stream>>>(qpart, wl.nqb, part, wl.grid, ln_w, ln_b, Wr, dWr,
-                                                                                  dbr, dln_w, dln_b, dnoise_scale, Dm, E);
+        AB_LAUNCH_CHECK();
+    }
+    const int G = param_groups(E);
+    router_param_kernel<<<(unsigned)ab_ceil_div(Dm, 32), dim3(32, E, G), 0, stream>>>(qpart, nqb, part, nparts, ln_w, ln_b, Wr, dWr,
+                                                                                     dbr, dln_w, dln_b, dnoise_scale, Dm, E);
     AB_LAUNCH_CHECK();
     return AB_OK;
 }
