@@ -988,6 +988,8 @@ extern "C" int ab_moe_router_fwd(const void* x, const float* ln_w, const float* 
     AB_REQUIRE(ws && ws_bytes >= wl.total, "moe_router_fwd: workspace too small");
     AB_REQUIRE(noise == nullptr || noise_scale != nullptr, "moe_router_fwd: noise without noise_scale");
     AB_REQUIRE(quant == AB_ROUTER_EXACT || quant == AB_ROUTER_BF16 || quant == AB_ROUTER_FP16, "moe_router_fwd: bad logit rounding mode %d", quant);
+    // modules.py::router_smem_bytes mirrors this size: AdaptiveExpertSystem refuses, at construction, hidden sizes
+    // whose router forward would not fit in a block's shared memory.  Change the two together.
     const size_t smem = ((size_t)E * Dm + 32 + WARPS * (2 * E + 1) + 2 * (size_t)Dm) * sizeof(float);
     float* part = (float*)ws;
     const int V = dtype == AB_F32 ? 4 : 8;

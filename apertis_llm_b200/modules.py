@@ -166,6 +166,21 @@ class SelectiveLinearAttention(nn.Module):
 # ================================================================================================
 # MoE layer
 # ================================================================================================
+# The router forward (csrc/moe_router.cu, ab_moe_router_fwd) keeps the router weight, its bias, the per-warp aux sums of
+# its 8 warps and the LayerNorm affine in dynamic shared memory, all fp32.  An sm_100 block can opt in to at most 227 KB.
+ROUTER_SMEM_LIMIT = 232448
+
+
+def router_smem_bytes(E: int, Dm: int) -> int:
+    """Dynamic shared memory of the router forward: (E*Dm + 32 + 8*(2E+1) + 2*Dm) floats."""
+    return (E * Dm + 32 + 8 * (2 * E + 1) + 2 * Dm) * 4
+
+
+def router_max_hidden(E: int) -> int:
+    """Largest hidden size (a multiple of 8) whose router forward fits in ROUTER_SMEM_LIMIT for E experts."""
+    return (ROUTER_SMEM_LIMIT // 4 - 32 - 8 * (2 * E + 1)) // (E + 2) // 8 * 8
+
+
 class AdaptiveExpertSystem(nn.Module):
     """B200-native AdaptiveExpertSystem (core.py:403-607).
 
@@ -199,6 +214,10 @@ class AdaptiveExpertSystem(nn.Module):
             raise ValueError(f"the B200 MoE kernels support num_experts <= 32 and experts_per_token <= 8 (got {E}, {self.experts_per_token})")
         if Dm % 8 or I % 8:
             raise ValueError(f"hidden_size ({Dm}) and intermediate_size ({I}) must be multiples of 8 (16-byte rows for TMA)")
+        if router_smem_bytes(E, Dm) > ROUTER_SMEM_LIMIT:
+            raise ValueError(f"the B200 router kernels stage the {E} x {Dm} router weight in shared memory: "
+                             f"{router_smem_bytes(E, Dm)} bytes exceed the {ROUTER_SMEM_LIMIT} a block can hold, so with "
+                             f"{E} experts hidden_size must be <= {router_max_hidden(E)}")
         if not 0.0 <= float(g("hidden_dropout_prob", 0.0)) < 1.0:
             raise ValueError("hidden_dropout_prob must be in [0, 1)")
         self.eps = config.layer_norm_eps
