@@ -108,7 +108,7 @@ struct RoundsParams {
     const float *dt_bias, *A_log, *D, *h0;
     float* h_last;
     float* hck;        // [B, nck8, Di]     state entering every group of 8 tokens
-    float* delta;      // [B, nslab, L8, 4] softplus(dt) of the slab's four heads
+    float* delta;      // [B, nslab, L8, 4] softplus(dt) of the slab's HPS <= 4 heads (unused slots hold 0)
     float4* agg;       // [2][nchains][cpr][32]   chunk aggregate (P0, P1, S0, S1) per lane; level 1 rewrites it as the exclusive prefix inside the segment
     float4* segagg;    // [2][nchains][nseg][32]
     float2* segcarry;  // [2][nchains][nseg][32]  state entering each segment
@@ -119,7 +119,8 @@ struct RoundsParams {
     unsigned* done;    // teams that have finished; the last one zeroes the counters for the next launch
     int cnt_words, nteams_used;
     float4* part;      // backward: [nw_used][32]  (dA0, dA1, dD0, dD1) accumulated by each warp over its chunks
-    float* part_b;     // backward: [nw_used][32]  d dt_bias share of lane (head lane >> 3, token lane & 7)
+    float* part_b;     // backward: [nw_used][32]  d dt_bias share of lane (head lane / (32 / HPS), token lane & 7); zero in
+                       //           the lanes of a head past its first 8
     int ddlog_cols;    // backward: columns [H, ddlog_cols) of the d dlog rows are written as zero (padding of a fused buffer)
 };
 
@@ -363,12 +364,12 @@ __device__ __forceinline__ void team_finish(const RoundsParams& p, int member, i
 // ====================================================================================================================
 template <typename T>
 struct FwdCtx {
-    const T* dlog;     // this lane's (token lane >> 2, head lane & 3) column of row 0 of the sequence
-    float* delta;      // this (sequence, slab)'s [L8, 4] block + head (lane & 3)
+    const T* dlog;     // this lane's (token lane >> 2, head slot lane & 3) column of row 0 of the sequence
+    float* delta;      // this (sequence, slab)'s [L8, 4] block + head slot (lane & 3)
     float* hck;        // this sequence's [nck8, Di] block + channel pair
     f2 A2, Dv;
     float bias;        // dt bias of the head this lane computes delta for
-    bool hv;           // head (lane & 3) valid
+    bool hv;           // head slot (lane & 3) holds a head: slot < HPS and head < H
     int L;
 };
 
@@ -423,7 +424,7 @@ __device__ __forceinline__ float dlog_fetch(const FwdCtx<T>& c, const Who& w, in
     const int tok = tb + (w.lane >> 2);
     return (w.real && c.hv && tb < tend && tok < c.L) ? ab_to_float(c.dlog[(int64_t)tok * dls]) : -1e30f;
 }
-// delta of 8 tokens x 4 heads, one (token, head) per lane; saved for P2 and the backward
+// delta of 8 tokens x 4 head slots, one (token, slot) per lane; saved for P2 and the backward
 template <typename T>
 __device__ __forceinline__ float delta_finish(const FwdCtx<T>& c, const Who& w, float raw, int tb, int tend) {
     const float d = raw > -1e29f ? ab_softplus_fast(raw + c.bias) : 0.f;
@@ -431,11 +432,11 @@ __device__ __forceinline__ float delta_finish(const FwdCtx<T>& c, const Who& w, 
     return d;
 }
 
-template <typename T, int TS, int NST, typename Feeder>
+template <typename T, int TS, int NST, int HPS, typename Feeder>
 __device__ __forceinline__ void fwd_p1(const RoundsParams& p, const FwdCtx<T>& c, const Who& w, Pipe& pp, Feeder& fd, const Cursor<false>& ph, f2 init) {
     const int t0 = ph.t0, tend = ph.tend, npieces = ph.n;
     const int dls = p.dlog_stride;
-    const int hsel = w.lane >> 3;
+    const int hsel = w.lane / (32 / HPS);
     f2 S = f2_bcast(0.f);
     float sumd = 0.f;
     float raw[4];
@@ -473,11 +474,11 @@ __device__ __forceinline__ void fwd_p1(const RoundsParams& p, const FwdCtx<T>& c
     publish_and_prefix(p, ph.r, w.chain, w.slot, ph.n_r, w.lane, P, S, init, fin);
 }
 
-template <typename T, bool YSSM, int TS, int NST, typename Feeder>
+template <typename T, bool YSSM, int TS, int NST, int HPS, typename Feeder>
 __device__ __forceinline__ void fwd_p2(const RoundsParams& p, const FwdCtx<T>& c, const Who& w, Pipe& pp, Feeder& fd, const FwdMaps& m,
                                        const Cursor<false>& ph, uint64_t pol_stream) {
     const int t0 = ph.t0, ngroups = ph.n, r = ph.r;
-    const int hsel = w.lane >> 3;
+    const int hsel = w.lane / (32 / HPS);
     constexpr int TB = Tile<T, TS>::BYTES;
     const float* dsrc = c.delta + (int64_t)(t0 + (w.lane >> 2)) * 4;
     float dnext = w.real ? __ldcg(dsrc) : 0.f;
@@ -556,7 +557,7 @@ __device__ __forceinline__ void who_am_i(const RoundsParams& p, Who& w, Pipe& pp
     __syncthreads();
 }
 
-template <typename T, bool YSSM, int TS, int NST>
+template <typename T, bool YSSM, int TS, int NST, int HPS>
 __global__ void __launch_bounds__(sizeof(T) == 2 ? 768 : 512, 1)
 scan_rounds_fwd_kernel(const __grid_constant__ CUtensorMap tm_xa, const __grid_constant__ CUtensorMap tm_b, const __grid_constant__ CUtensorMap tm_b32,
                        const __grid_constant__ CUtensorMap tm_c, const __grid_constant__ CUtensorMap tm_z, const __grid_constant__ CUtensorMap tm_y,
@@ -570,7 +571,8 @@ scan_rounds_fwd_kernel(const __grid_constant__ CUtensorMap tm_xa, const __grid_c
     const int c0 = w.slab * 64 + 2 * lane;
     FwdCtx<T> c;
     c.L = p.L;
-    const int head = w.slab * 4 + (lane & 3);
+    // head slots past the slab's HPS heads get head H (invalid): one test in the loops, not two
+    const int head = (HPS == 4 || (lane & 3) < HPS) ? w.slab * HPS + (lane & 3) : p.H;
     c.hv = w.real && head < p.H;
     c.bias = (c.hv && p.dt_bias != nullptr) ? p.dt_bias[head] : 0.f;
     const int cs = w.cv ? c0 : 0;
@@ -587,8 +589,8 @@ scan_rounds_fwd_kernel(const __grid_constant__ CUtensorMap tm_xa, const __grid_c
     if (w.leader) fd.prime();
     Cursor<false> ph;
     for (ph.begin(p, w.slot); ph.kind >= 0; ph.next_phase(p, w.slot)) {
-        if (ph.kind == 0) fwd_p1<T, TS, NST>(p, c, w, pp, fd, ph, init);
-        else fwd_p2<T, YSSM, TS, NST>(p, c, w, pp, fd, m, ph, pol_stream);
+        if (ph.kind == 0) fwd_p1<T, TS, NST, HPS>(p, c, w, pp, fd, ph, init);
+        else fwd_p2<T, YSSM, TS, NST, HPS>(p, c, w, pp, fd, m, ph, pol_stream);
     }
     if (w.leader) bulk_wait_all();
     team_finish(p, w.member, w.lane);
@@ -662,10 +664,10 @@ struct BwdFeeder {
     }
 };
 
-template <typename T, bool YSSM, int TS, int NST, typename Feeder>
+template <typename T, bool YSSM, int TS, int NST, int HPS, typename Feeder>
 __device__ __forceinline__ void bwd_p1(const RoundsParams& p, const BwdCtx<T>& c, const Who& w, Pipe& pp, Feeder& fd, const Cursor<true>& ph) {
     const int t0 = ph.t0, ngroups = ph.n;          // groups are visited last to first: step i handles group ngroups - 1 - i
-    const int hsel = w.lane >> 3;
+    const int hsel = w.lane / (32 / HPS);
     f2 F = f2_bcast(0.f);
     float sumd = 0.f;
     const float* dsrc = c.delta + (int64_t)(t0 + (ngroups - 1) * RG + (w.lane >> 2)) * 4;
@@ -696,11 +698,12 @@ __device__ __forceinline__ void bwd_p1(const RoundsParams& p, const BwdCtx<T>& c
     publish_and_prefix(p, ph.r, w.chain, w.slot, ph.n_r, w.lane, P, F, f2_bcast(0.f), nullptr);
 }
 
-template <typename T, bool YSSM, int TS, int NST, typename Feeder>
+template <typename T, bool YSSM, int TS, int NST, int HPS, typename Feeder>
 __device__ __forceinline__ void bwd_p2(const RoundsParams& p, const BwdCtx<T>& c, const Who& w, Pipe& pp, Feeder& fd, const BwdMaps& m,
                                        const Cursor<true>& ph, f2& accA, f2& accD, float& accB, uint64_t pol_stream) {
     const int t0 = ph.t0, ngroups = ph.n, r = ph.r;
-    const int hsel = w.lane >> 3;
+    constexpr int LPH = 32 / HPS;                  // lanes per head
+    const int hsel = w.lane / LPH;
     constexpr int TB = Tile<T, TS>::BYTES;
     const float* hck = c.hck + (size_t)((t0 >> 3) + ngroups - 1) * p.Di;
     const float* dsrc = c.delta + (int64_t)(t0 + (ngroups - 1) * RG + (w.lane >> 2)) * 4;
@@ -770,8 +773,9 @@ __device__ __forceinline__ void bwd_p2(const RoundsParams& p, const BwdCtx<T>& c
             bulk_commit();
         }
         ++pp.k;
-        // ---- d delta: sum over the 8 lanes of a head (16 channels), transposing butterfly over the 8 tokens so that lane
-        //      (head hsel, k = lane & 7) ends with the total of token k
+        // ---- d delta: transposing butterfly over the 8 tokens inside each group of 8 lanes (16 channels), so that lane
+        //      (head hsel, k = lane & 7) holds its group's share of token k, then the sum over the LPH / 8 groups of the head;
+        //      every lane of a head then holds the same totals and only its first 8 lanes write them
         {
             const int k = w.lane & 7;
             float s4[4];
@@ -790,25 +794,29 @@ __device__ __forceinline__ void bwd_p2(const RoundsParams& p, const BwdCtx<T>& c
             }
             const float keep = (k & 1) ? s2[1] : s2[0];
             const float send = (k & 1) ? s2[0] : s2[1];
-            const float tot = keep + __shfl_xor_sync(0xffffffffu, send, 1);      // token k of head hsel
+            float tot = keep + __shfl_xor_sync(0xffffffffu, send, 1);            // token k of head hsel
+#pragma unroll
+            for (int m = 8; m < LPH; m <<= 1) tot += __shfl_xor_sync(0xffffffffu, tot, m);
             const float dk = __shfl_sync(0xffffffffu, dmine, k * 4 + hsel);       // delta of (token k, head hsel)
-            const int head = w.slab * 4 + hsel;
+            const int head = w.slab * HPS + hsel;
             const int tok = tb + k;
-            if (w.real && tok < c.L) {
+            if (w.real && tok < c.L && (w.lane & (LPH - 1)) < 8) {
                 if (head < p.H) {
                     // softplus'(x) = sigmoid(x) = 1 - exp(-softplus(x))
                     const float gq = tot * (1.0f - ab_ex2(-dk * AB_LOG2E));
                     accB += gq;
                     c.ddlog[(int64_t)tok * p.ddlog_stride + head] = ab_from_float<T>(gq);
                 }
-                for (int hh = head; hh < p.ddlog_cols; hh += 4)       // padding columns (covered by the last slab's lanes)
+                int hh = head;
+                if constexpr (HPS < 4) { if (hh < p.H) hh += (p.H - hh + HPS - 1) / HPS * HPS; }      // first padding column of this head's class
+                for (; hh < p.ddlog_cols; hh += HPS)     // padding columns (covered by the last slab's lanes)
                     if (hh >= p.H) c.ddlog[(int64_t)tok * p.ddlog_stride + hh] = ab_from_float<T>(0.f);
             }
         }
     }
 }
 
-template <typename T, bool YSSM, int TS, int NST>
+template <typename T, bool YSSM, int TS, int NST, int HPS>
 __global__ void __launch_bounds__(sizeof(T) == 2 ? 512 : 256, 1)
 scan_rounds_bwd_kernel(const __grid_constant__ CUtensorMap tm_xa, const __grid_constant__ CUtensorMap tm_b, const __grid_constant__ CUtensorMap tm_c,
                        const __grid_constant__ CUtensorMap tm_z, const __grid_constant__ CUtensorMap tm_g, const __grid_constant__ CUtensorMap tm_s,
@@ -840,8 +848,8 @@ scan_rounds_bwd_kernel(const __grid_constant__ CUtensorMap tm_xa, const __grid_c
     if (w.leader) fd.prime();
     Cursor<true> ph;
     for (ph.begin(p, w.slot); ph.kind >= 0; ph.next_phase(p, w.slot)) {
-        if (ph.kind == 0) bwd_p1<T, YSSM, TS, NST>(p, c, w, pp, fd, ph);
-        else bwd_p2<T, YSSM, TS, NST>(p, c, w, pp, fd, m, ph, accA, accD, accB, pol_stream);
+        if (ph.kind == 0) bwd_p1<T, YSSM, TS, NST, HPS>(p, c, w, pp, fd, ph);
+        else bwd_p2<T, YSSM, TS, NST, HPS>(p, c, w, pp, fd, m, ph, accA, accD, accB, pol_stream);
     }
     if (w.leader) bulk_wait_all();
     {
@@ -861,6 +869,7 @@ scan_rounds_bwd_kernel(const __grid_constant__ CUtensorMap tm_xa, const __grid_c
 // (eight loads in flight per lane); the CTA that finishes last adds the RED_SPLIT shares in index order.
 constexpr int RED_SPLIT = 8;
 
+template <int HPS>
 __global__ void __launch_bounds__(256) scan_rounds_param_reduce_kernel(const float4* __restrict__ part, const float* __restrict__ part_b, float* __restrict__ dA,
                                                                         float* __restrict__ dD, float* __restrict__ dbias, float4* __restrict__ stage2,
                                                                         float* __restrict__ stage2_b, unsigned* __restrict__ arrive, int Di, int H, int B,
@@ -923,12 +932,12 @@ __global__ void __launch_bounds__(256) scan_rounds_param_reduce_kernel(const flo
             }
             const int c0 = slab * 64 + 2 * lane;
             if (c0 < Di) { dA[c0] = tot.x; dA[c0 + 1] = tot.y; dD[c0] = tot.z; dD[c0 + 1] = tot.w; }
-            // lanes (head lane >> 3, token lane & 7): sum the 8 token lanes of a head
+            // lanes (head lane / (32 / HPS), token lane & 7): sum the 8 token lanes of a head (its other lanes hold zeros)
             tb2 += __shfl_xor_sync(0xffffffffu, tb2, 4);
             tb2 += __shfl_xor_sync(0xffffffffu, tb2, 2);
             tb2 += __shfl_xor_sync(0xffffffffu, tb2, 1);
-            const int head = slab * 4 + (lane >> 3);
-            if (dbias != nullptr && (lane & 7) == 0 && head < H) dbias[head] = tb2;
+            const int head = slab * HPS + lane / (32 / HPS);
+            if (dbias != nullptr && (lane & (32 / HPS - 1)) == 0 && head < H) dbias[head] = tb2;
         }
     }
 }
@@ -1047,9 +1056,13 @@ void fill_sync(RoundsParams& p, const RoundsCfg& c, void* ws) {
 
 int g_tc_hint_fwd = 0, g_tc_hint_bwd = 0, g_warp_cap = 0;
 
+// A 64-channel slab holds 64 / N whole heads of N = Di / H channels (ssm_d_state); N = 16, 32, 64 -> 4, 2, 1 heads per slab.
+int heads_per_slab(int Di, int H) { return 64 * H / Di; }
+
 int common_checks(const char* who, int B, int L, int Di, int H, int dtype) {
     AB_REQUIRE(B > 0 && L > 0 && Di > 0 && H > 0, "%s: B, L, Di, H must be positive", who);
-    AB_REQUIRE(Di == 16 * H, "%s: Di (%d) must equal 16 * H (%d): the kernel is specialised for ssm_d_state 16", who, Di, H);
+    AB_REQUIRE(Di == 16 * H || Di == 32 * H || Di == 64 * H,
+               "%s: Di (%d) must be N * H (H = %d) with ssm_d_state N in {16, 32, 64}", who, Di, H);
     AB_REQUIRE(dtype == AB_F32 || dtype == AB_BF16, "%s: bad dtype %d", who, dtype);
     return AB_OK;
 }
@@ -1099,55 +1112,71 @@ int set_smem(K kernel, size_t bytes) {
 struct FwdLaunch {
     CUtensorMap xa, b, b32, c, z, y, ys;
 };
-template <typename T, bool YS, int TS, int NST>
+template <typename T, bool YS, int TS, int NST, int HPS>
 int launch_fwd_n(const FwdLaunch& m, const RoundsParams& p, const RoundsCfg& c, cudaStream_t stream) {
     static size_t configured = 0;          // cudaFuncSetAttribute is a driver call: only when the requirement grows
     if (c.smem > configured) {
-        if (int e = set_smem(scan_rounds_fwd_kernel<T, YS, TS, NST>, c.smem)) return e;
+        if (int e = set_smem(scan_rounds_fwd_kernel<T, YS, TS, NST, HPS>, c.smem)) return e;
         configured = c.smem;
     }
-    scan_rounds_fwd_kernel<T, YS, TS, NST><<<c.grid, c.block, c.smem, stream>>>(m.xa, m.b, m.b32, m.c, m.z, m.y, m.ys, p);
+    scan_rounds_fwd_kernel<T, YS, TS, NST, HPS><<<c.grid, c.block, c.smem, stream>>>(m.xa, m.b, m.b32, m.c, m.z, m.y, m.ys, p);
     AB_LAUNCH_CHECK();
     return AB_OK;
 }
-template <typename T, bool YS, int TS>
+template <typename T, bool YS, int TS, int HPS>
 int launch_fwd(const FwdLaunch& m, const RoundsParams& p, const RoundsCfg& c, cudaStream_t stream) {
-    return c.NST == 3 ? launch_fwd_n<T, YS, TS, 3>(m, p, c, stream) : launch_fwd_n<T, YS, TS, 2>(m, p, c, stream);
+    return c.NST == 3 ? launch_fwd_n<T, YS, TS, 3, HPS>(m, p, c, stream) : launch_fwd_n<T, YS, TS, 2, HPS>(m, p, c, stream);
 }
-template <typename T, bool YS>
+template <typename T, bool YS, int HPS>
 int launch_fwd_ts(const FwdLaunch& m, const RoundsParams& p, const RoundsCfg& c, cudaStream_t stream) {
     switch (c.TS) {
-        case 1: return launch_fwd<T, YS, 1>(m, p, c, stream);
-        case 2: return launch_fwd<T, YS, 2>(m, p, c, stream);
-        case 3: return launch_fwd<T, YS, 3>(m, p, c, stream);
-        default: return launch_fwd<T, YS, 4>(m, p, c, stream);
+        case 1: return launch_fwd<T, YS, 1, HPS>(m, p, c, stream);
+        case 2: return launch_fwd<T, YS, 2, HPS>(m, p, c, stream);
+        case 3: return launch_fwd<T, YS, 3, HPS>(m, p, c, stream);
+        default: return launch_fwd<T, YS, 4, HPS>(m, p, c, stream);
+    }
+}
+template <typename T, bool YS>
+int launch_fwd_hps(const FwdLaunch& m, const RoundsParams& p, const RoundsCfg& c, int hps, cudaStream_t stream) {
+    switch (hps) {
+        case 4: return launch_fwd_ts<T, YS, 4>(m, p, c, stream);
+        case 2: return launch_fwd_ts<T, YS, 2>(m, p, c, stream);
+        default: return launch_fwd_ts<T, YS, 1>(m, p, c, stream);
     }
 }
 struct BwdLaunch {
     CUtensorMap xa, b, c, z, g, s, dxa, db, dc, dz;
 };
-template <typename T, bool YS, int TS, int NST>
+template <typename T, bool YS, int TS, int NST, int HPS>
 int launch_bwd_n(const BwdLaunch& m, const RoundsParams& p, const RoundsCfg& c, cudaStream_t stream) {
     static size_t configured = 0;
     if (c.smem > configured) {
-        if (int e = set_smem(scan_rounds_bwd_kernel<T, YS, TS, NST>, c.smem)) return e;
+        if (int e = set_smem(scan_rounds_bwd_kernel<T, YS, TS, NST, HPS>, c.smem)) return e;
         configured = c.smem;
     }
-    scan_rounds_bwd_kernel<T, YS, TS, NST><<<c.grid, c.block, c.smem, stream>>>(m.xa, m.b, m.c, m.z, m.g, m.s, m.dxa, m.db, m.dc, m.dz, p);
+    scan_rounds_bwd_kernel<T, YS, TS, NST, HPS><<<c.grid, c.block, c.smem, stream>>>(m.xa, m.b, m.c, m.z, m.g, m.s, m.dxa, m.db, m.dc, m.dz, p);
     AB_LAUNCH_CHECK();
     return AB_OK;
 }
-template <typename T, bool YS, int TS>
+template <typename T, bool YS, int TS, int HPS>
 int launch_bwd(const BwdLaunch& m, const RoundsParams& p, const RoundsCfg& c, cudaStream_t stream) {
-    return c.NST == 3 ? launch_bwd_n<T, YS, TS, 3>(m, p, c, stream) : launch_bwd_n<T, YS, TS, 2>(m, p, c, stream);
+    return c.NST == 3 ? launch_bwd_n<T, YS, TS, 3, HPS>(m, p, c, stream) : launch_bwd_n<T, YS, TS, 2, HPS>(m, p, c, stream);
 }
-template <typename T, bool YS>
+template <typename T, bool YS, int HPS>
 int launch_bwd_ts(const BwdLaunch& m, const RoundsParams& p, const RoundsCfg& c, cudaStream_t stream) {
     switch (c.TS) {
-        case 1: return launch_bwd<T, YS, 1>(m, p, c, stream);
-        case 2: return launch_bwd<T, YS, 2>(m, p, c, stream);
-        case 3: return launch_bwd<T, YS, 3>(m, p, c, stream);
-        default: return launch_bwd<T, YS, 4>(m, p, c, stream);
+        case 1: return launch_bwd<T, YS, 1, HPS>(m, p, c, stream);
+        case 2: return launch_bwd<T, YS, 2, HPS>(m, p, c, stream);
+        case 3: return launch_bwd<T, YS, 3, HPS>(m, p, c, stream);
+        default: return launch_bwd<T, YS, 4, HPS>(m, p, c, stream);
+    }
+}
+template <typename T, bool YS>
+int launch_bwd_hps(const BwdLaunch& m, const RoundsParams& p, const RoundsCfg& c, int hps, cudaStream_t stream) {
+    switch (hps) {
+        case 4: return launch_bwd_ts<T, YS, 4>(m, p, c, stream);
+        case 2: return launch_bwd_ts<T, YS, 2>(m, p, c, stream);
+        default: return launch_bwd_ts<T, YS, 1>(m, p, c, stream);
     }
 }
 
@@ -1208,8 +1237,9 @@ extern "C" int ab_ssm_scan_fwd(const void* xa, int64_t xa_stride, const void* dl
     if (int e = map3(&m.y, y, dtype, B, L, Di, Di, RG, cols)) return e;
     m.ys = m.y;
     if (y_ssm) { if (int e = map3(&m.ys, y_ssm, dtype, B, L, Di, Di, RG, cols)) return e; }
-    if (dtype == AB_F32) return y_ssm ? launch_fwd_ts<float, true>(m, p, c, stream) : launch_fwd_ts<float, false>(m, p, c, stream);
-    return y_ssm ? launch_fwd_ts<__nv_bfloat16, true>(m, p, c, stream) : launch_fwd_ts<__nv_bfloat16, false>(m, p, c, stream);
+    const int hps = heads_per_slab(Di, H);
+    if (dtype == AB_F32) return y_ssm ? launch_fwd_hps<float, true>(m, p, c, hps, stream) : launch_fwd_hps<float, false>(m, p, c, hps, stream);
+    return y_ssm ? launch_fwd_hps<__nv_bfloat16, true>(m, p, c, hps, stream) : launch_fwd_hps<__nv_bfloat16, false>(m, p, c, hps, stream);
 }
 
 extern "C" int ab_ssm_scan_bwd(const void* xa, int64_t xa_stride, const void* Bm, const void* Cm, int64_t bc_stride,
@@ -1252,16 +1282,17 @@ extern "C" int ab_ssm_scan_bwd(const void* xa, int64_t xa_stride, const void* Bm
     if (int e = map3(&m.db, dBm, dtype, B, L, Di, dbc_stride, RG, cols)) return e;
     if (int e = map3(&m.dc, dCm, dtype, B, L, Di, dbc_stride, RG, cols)) return e;
     if (int e = map3(&m.dz, dz, dtype, B, L, Di, dz_stride, RG, cols)) return e;
+    const int hps = heads_per_slab(Di, H);
     int e;
-    if (dtype == AB_F32) e = dyssm ? launch_bwd_ts<float, true>(m, p, c, stream) : launch_bwd_ts<float, false>(m, p, c, stream);
-    else e = dyssm ? launch_bwd_ts<__nv_bfloat16, true>(m, p, c, stream) : launch_bwd_ts<__nv_bfloat16, false>(m, p, c, stream);
+    if (dtype == AB_F32) e = dyssm ? launch_bwd_hps<float, true>(m, p, c, hps, stream) : launch_bwd_hps<float, false>(m, p, c, hps, stream);
+    else e = dyssm ? launch_bwd_hps<__nv_bfloat16, true>(m, p, c, hps, stream) : launch_bwd_hps<__nv_bfloat16, false>(m, p, c, hps, stream);
     if (e) return e;
     unsigned char* w8 = reinterpret_cast<unsigned char*>(ws);
     float4* stage2 = reinterpret_cast<float4*>(w8 + c.off_stage2);
     float* stage2_b = reinterpret_cast<float*>(stage2 + (size_t)c.nslab * RED_SPLIT * 32);
-    scan_rounds_param_reduce_kernel<<<dim3(c.nslab, RED_SPLIT), 256, 0, stream>>>(p.part, p.part_b, dA_log, dD, ddt_bias, stage2, stage2_b,
-                                                                              reinterpret_cast<unsigned*>(w8 + 64), Di, H, B, c.TS, c.tps,
-                                                                              c.nteamchains, c.cpr);
+    auto reduce = hps == 4 ? scan_rounds_param_reduce_kernel<4> : hps == 2 ? scan_rounds_param_reduce_kernel<2> : scan_rounds_param_reduce_kernel<1>;
+    reduce<<<dim3(c.nslab, RED_SPLIT), 256, 0, stream>>>(p.part, p.part_b, dA_log, dD, ddt_bias, stage2, stage2_b, reinterpret_cast<unsigned*>(w8 + 64),
+                                                         Di, H, B, c.TS, c.tps, c.nteamchains, c.cpr);
     AB_LAUNCH_CHECK();
     return AB_OK;
 }

@@ -76,6 +76,10 @@ def _compute_dtype(ac: Optional[torch.dtype]) -> Optional[torch.dtype]:
 # ================================================================================================
 # SSM layer
 # ================================================================================================
+SSM_D_STATES = (16, 32, 64)              # ssm_d_state values the selective-scan kernels take (csrc/ssm_scan_rounds.cu)
+SSM_CONV_KERNELS = tuple(range(2, 9))    # ssm_conv_kernel values the causal-conv kernels take (csrc/ssm_conv.cu)
+
+
 class SelectiveLinearAttention(nn.Module):
     """B200-native SelectiveLinearAttention (core.py:295-401): same parameters, same forward contract."""
 
@@ -87,8 +91,13 @@ class SelectiveLinearAttention(nn.Module):
         self.d_inner = self.num_heads * self.d_state
         self.dt_rank = config.ssm_dt_rank
         self.conv_kernel_size = config.ssm_conv_kernel
-        if self.d_state != 16:
-            raise NotImplementedError("the selective-scan kernel is specialised for ssm_d_state == 16 (the reference default)")
+        # limits of the kernels: a 64-channel slab of the scan holds whole heads; the conv keeps its window in registers.
+        # ssm_conv_kernel 1 stays out: the reference's conv state x_seq[:, :, -(Kc-1):] (core.py:372) is then the whole sequence
+        if self.d_state not in SSM_D_STATES:
+            raise NotImplementedError(f"the selective-scan kernels support ssm_d_state in {SSM_D_STATES} (got {self.d_state})")
+        if not SSM_CONV_KERNELS[0] <= self.conv_kernel_size <= SSM_CONV_KERNELS[-1]:
+            raise NotImplementedError(f"the causal-conv kernels support ssm_conv_kernel in {SSM_CONV_KERNELS[0]}..{SSM_CONV_KERNELS[-1]} "
+                                      f"(got {self.conv_kernel_size})")
         self.in_proj_x = nn.Linear(self.hidden_size, self.d_inner, bias=False)
         self.in_proj_z = nn.Linear(self.hidden_size, self.d_inner, bias=False)
         self.conv1d = nn.Conv1d(self.d_inner, self.d_inner, kernel_size=self.conv_kernel_size, groups=self.d_inner,

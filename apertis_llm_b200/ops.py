@@ -253,7 +253,7 @@ class _CausalConv1dSiLU(torch.autograd.Function):
 
 
 def causal_conv1d_silu(xp: torch.Tensor, weight: torch.Tensor, bias: torch.Tensor) -> torch.Tensor:
-    """xp [B,L,Di] (channels last), weight [Di,1,4], bias [Di] -> silu(causal depthwise conv) [B,L,Di]."""
+    """xp [B,L,Di] (channels last), weight [Di,1,Kc] (2 <= Kc <= 8), bias [Di] -> silu(causal depthwise conv) [B,L,Di]."""
     return _CausalConv1dSiLU.apply(xp, weight, bias)
 
 

@@ -52,7 +52,8 @@ int ab_device_check(int device);
 int ab_last_error(char* buf, size_t n);
 
 /* ---- SSM: causal depthwise conv1d + SiLU  (core.py:368-375) ----------------------------------
- * xa[b,t,c] = silu(bias[c] + sum_j w[c,j] * xp[b,t-(Kc-1)+j,c]), zero left padding.  Kc must be 4.
+ * xa[b,t,c] = silu(bias[c] + sum_j w[c,j] * xp[b,t-(Kc-1)+j,c]), zero left padding.  2 <= Kc <= 8.
+ * The backward workspace (ab_causal_conv1d_silu_bwd_workspace_bytes) is sized for Kc = 8, so it serves every Kc.
  * xp rows may be strided (xp_stride elements between tokens); xa is contiguous [B,L,Di]. */
 int ab_causal_conv1d_silu_fwd(const void* xp, int64_t xp_stride, const float* w, const float* bias, void* xa,
                               int B, int L, int Di, int Kc, int dtype, cudaStream_t stream);
@@ -121,8 +122,9 @@ int ab_dt_compose_bwd(const float* dWcat, const float* Wp, const float* Wdt, flo
                       int R, int Di, cudaStream_t stream);
 
 /* ---- SSM: selective scan, "rounds" schedule (csrc/ssm_scan_rounds.cu) ------------------------------------------
- * Same arithmetic as above (core.py:324-353, :383, :394-396), one persistent kernel per direction: warps walk chunks of
- * one 64-channel slab serially (two channels per lane), every chunk is visited twice (aggregate pass, then the streaming
+ * Same arithmetic as above (core.py:324-353, :383, :394-396) for channel c = h*N + n with ssm_d_state N = Di / H in
+ * {16, 32, 64} (the older schedules above take N = 16 only), one persistent kernel per direction: warps walk chunks of
+ * one 64-channel slab (4, 2 or 1 whole heads) serially (two channels per lane), every chunk is visited twice (aggregate pass, then the streaming
  * pass with the incoming state known), a round's chunk aggregates are prefixed by a two-level scan of whoever arrives
  * last.  Row strides are in elements; every activation may be a column slice of a wider row-major buffer, which is how
  * the fused projection outputs ([xp | z] and [dt | B | C]) are consumed and produced without copies.

@@ -3,6 +3,7 @@
 kernels forward + backward, seq 2K..64K, HBM GB/s against the algorithmic bytes of SURVEY.md section 8(d).
 
     python tools/scan_bench.py [--dtype bf16|f32] [--mode rounds|pipe|single|two_pass] [--seqs 2048,...] [--batch 1] [--iters 20]
+                               [--heads 32] [--d-state 16]     (Di = d_state * heads; the older modes take d_state 16 only)
 """
 import argparse
 import json
@@ -27,6 +28,7 @@ def main():
     ap.add_argument("--seqs", default="2048,4096,8192,16384,32768,65536")
     ap.add_argument("--batch", type=int, default=1)
     ap.add_argument("--heads", type=int, default=32)
+    ap.add_argument("--d-state", type=int, default=16, help="ssm_d_state N: 16, 32 or 64 (Di = N * heads)")
     ap.add_argument("--iters", type=int, default=20)
     ap.add_argument("--json", default="")
     ap.add_argument("--graph", action="store_true", help="time CUDA-graph replays of the launches (no host code inside the event windows)")
@@ -36,8 +38,8 @@ def main():
     es = 2 if dtype == torch.bfloat16 else 4
     mode = {"single": _lib.SCAN_SINGLE_PASS, "two_pass": _lib.SCAN_TWO_PASS, "pipe": _lib.SCAN_PIPELINED, "rounds": _lib.SCAN_ROUNDS}[args.mode]
     _lib.load().ab_ssm_scan_tune(args.tc_fwd, args.tc_bwd, args.wps, args.nst_fwd, args.nst_bwd)
-    H = args.heads
-    Di = 16 * H
+    H, N = args.heads, args.d_state
+    Di = N * H
     B = args.batch
     peak = 6539.2
     try:
@@ -51,7 +53,7 @@ def main():
         mk = lambda *s: torch.randn(*s, generator=g).to(d, dtype)
         xa, z, BC = mk(B, L, Di), mk(B, L, Di), mk(B, L, 2 * Di)
         dlog = (torch.randn(B, L, H, generator=g) - 3.0).to(d, dtype)
-        A_log = (torch.rand(H, 16, generator=g) * 0.68 - 0.69).to(d)
+        A_log = (torch.rand(H, N, generator=g) * 0.68 - 0.69).to(d)
         D = torch.ones(Di, device=d)
         dy = mk(B, L, Di)
         leaves = [t.requires_grad_(True) for t in (xa, dlog, BC, z)]
@@ -100,11 +102,11 @@ def main():
         mf, mb = tf[len(tf) // 2], tb[len(tb) // 2]
         tok = B * L
         bf, bb = tok * (5 * Di + H) * es, tok * (9 * Di + 2 * H) * es
-        rec = dict(L=L, B=B, dtype=args.dtype, mode=args.mode, fwd_us=mf * 1e3, bwd_us=mb * 1e3,
+        rec = dict(L=L, B=B, H=H, d_state=N, Di=Di, dtype=args.dtype, mode=args.mode, fwd_us=mf * 1e3, bwd_us=mb * 1e3,
                    fwd_gbs=bf / mf / 1e6, bwd_gbs=bb / mb / 1e6, fwdbwd_gbs=(bf + bb) / (mf + mb) / 1e6,
                    frac_of_measured_peak=(bf + bb) / (mf + mb) / 1e6 / peak, tokens_per_s=tok / ((mf + mb) * 1e-3))
         out.append(rec)
-        print(f"L={L:6d} fwd {mf * 1e3:8.1f} us {rec['fwd_gbs']:7.0f} GB/s | bwd {mb * 1e3:8.1f} us {rec['bwd_gbs']:7.0f} GB/s | "
+        print(f"L={L:6d} N={N:2d} fwd {mf * 1e3:8.1f} us {rec['fwd_gbs']:7.0f} GB/s | bwd {mb * 1e3:8.1f} us {rec['bwd_gbs']:7.0f} GB/s | "
               f"fwd+bwd {rec['fwdbwd_gbs']:7.0f} GB/s = {100 * rec['frac_of_measured_peak']:5.1f}% of {peak:.0f}")
     if args.json:
         json.dump(out, open(args.json, "w"), indent=1)
